@@ -18,6 +18,13 @@ line whose parity fails exits 1.
 
   python bench.py --gpus 1 --steps 20 --warmup 3
   python bench.py --impl reference ...   # the reference algorithm on host cores
+  python bench.py --dump-outputs DIR ... # also write the computed arrays as DIR/<name>.npy
+
+`--dump-outputs DIR` writes, in float64, what the timed path hands its caller: the level-0 iterate
+after the last timed V-cycle (`u_level0`); for micro8193, one damped-Jacobi sweep (`jacobi_sweep`)
+and one residual (`residual`) of the start iterate the timed launches work on.  A vector longer than
+2^21 entries is cut to a fixed, seeded sample of 2^21 of them (16 MB).  The inputs depend only on
+the arguments, so two builds run with the same arguments can be compared array for array.
 
 `--impl reference` times the reference's own V-cycle (symmetric Gauss-Seidel,
 /root/reference/include/amg/multigrid.hpp:263-305) as restated by the CPU oracle -- the
@@ -36,6 +43,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only: leave no __pycache__ in it
 
 WORKLOADS = {
     "vcycle4097": dict(n=4097, eps=1.0, smoother="jacobi"),
@@ -69,7 +77,15 @@ def parse_args():
     p.add_argument("--no-parity", action="store_true")
     p.add_argument("--no-cpu-baseline", action="store_true")
     p.add_argument("--no-e2e", action="store_true")
+    p.add_argument("--dump-outputs", metavar="DIR", default="",
+                   help="write the arrays the timed path computed in its last step as DIR/<name>.npy")
     a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        p.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
+    if a.dump_outputs and a.workload == "micro8193" and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        p.error("--dump-outputs: micro8193 writes its outputs on one GPU only")
     w = WORKLOADS[a.workload]
     a.n = a.n or w["n"]
     a.eps = a.eps or w["eps"]
@@ -151,6 +167,21 @@ class ClockSampler:
         return {"sm_mhz": sm[len(sm) // 2] if sm else None,
                 "sm_max_mhz": max(mx) if mx else None,
                 "samples": len(sm), "window": window, "reasons": sorted(reasons)}
+
+
+DUMP_SAMPLE = 1 << 21
+
+
+def dump_outputs(d, arrays):
+    """Write every array as d/<name>.npy in float64; one longer than DUMP_SAMPLE entries is cut to
+    the entries at DUMP_SAMPLE indices drawn with a fixed seed (the same indices for the same size)."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for name, x in arrays.items():
+        x = np.asarray(x, np.float64).reshape(-1)
+        if x.size > DUMP_SAMPLE:
+            x = x[np.sort(np.random.default_rng(0).choice(x.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(d, name + ".npy"), x)
 
 
 def measured_hbm_peak():
@@ -373,6 +404,11 @@ def run_b200(a):
     # one problem, row blocks spread over the ranks: whole-job V-cycles = steps
     vps = a.steps / (ms * 1e-3)
     rss_after = mg.rss()
+    if a.dump_outputs:
+        u_last = mg.get_soln(0)    # collective on >1 GPU: every rank takes part
+        if rank == 0:
+            dump_outputs(a.dump_outputs, {"u_level0": u_last})
+        del u_last
 
     # ---- e2e: host-resident b and u; H2D(b,u) + V-cycle + D2H(u) each step, through the C ABI.
     # On >1 GPU every rank owns the row block [r0, r1) of b and u (amgb_hierarchy_*_local): the
@@ -674,6 +710,8 @@ def run_micro(a, amg, rank, world, local, dist, comm, json_fd):
         r_cpu = O.five_point_residual(a.n, a.eps, u0, b)
         rel_res = float(np.linalg.norm(r_gpu - r_cpu) / np.linalg.norm(r_cpu))
         ok = ok and r_gpu.tobytes() == r_cpu.tobytes()
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, {"jacobi_sweep": got, "residual": r_gpu})
     if dist is not None:
         t = torch.tensor([1.0 if ok else 0.0], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MIN)
