@@ -22,6 +22,7 @@ SMOOTHER_GS, SMOOTHER_JACOBI, SMOOTHER_COLOR_GS = 0, 1, 2
 GS_AUTO, GS_LEVELSCHED, GS_LINESCAN = 0, 1, 2
 GS_KERNEL_FRONTS, GS_KERNEL_LINESCAN, GS_KERNEL_WAVE = 0, 1, 2
 ARITH_REFERENCE, ARITH_FAST = 0, 1
+TRANSFER_LINEAR, TRANSFER_BILINEAR_2D = 0, 1
 
 _i, _l, _d, _p = C.c_int, C.c_int64, C.c_double, C.c_void_p
 _pd = np.ctypeslib.ndpointer(dtype=np.float64, flags="C_CONTIGUOUS")
@@ -33,7 +34,8 @@ class Options(C.Structure):
                 ("compute_error_every_n_iters", _l), ("n_iters", _l),
                 ("smoother", _i), ("smoother_iters", _l), ("omega", _d),
                 ("gs_mode", _i), ("use_graph", _i),
-                ("skip_dead_coarse_smooth", _i), ("fuse", _i), ("arith", _i)]
+                ("skip_dead_coarse_smooth", _i), ("fuse", _i), ("arith", _i),
+                ("transfer", _i)]
 
 
 class AmgbError(RuntimeError):
@@ -60,6 +62,9 @@ SIGNATURES = {
     "amgb_n_H_dofs_from_n_h_dofs": (_l, [_l]),
     "amgb_interp_nnz": (_l, [_l, _l]),
     "amgb_interp_make_operators": (_i, [_l, _l, _pi, _pi, _pd, _pi, _pi, _pd]),
+    "amgb_bilinear_coarse_lines": (_l, [_l]),
+    "amgb_bilinear_nnz": (_l, [_l, _l]),
+    "amgb_bilinear_make_operators": (_i, [_l, _l, _pi, _pi, _pd, _pi, _pi, _pd]),
     "amgb_linear_restrict": (_i, [_l, _l, _pd, _pd]),
     "amgb_linear_prolong": (_i, [_l, _l, _pd, _pd]),
     "amgb_csc_spmv": (_i, [_i, _i, _pi, _pi, _pd, _pd, _pd]),
@@ -81,6 +86,7 @@ SIGNATURES = {
     "amgb_hierarchy_create": (_i, [_i, _i, _pi, _pi, _pd, _pd, _l, C.POINTER(Options),
                                    C.POINTER(_p)]),
     "amgb_hierarchy_destroy": (_i, [_p]),
+    "amgb_hierarchy_transfer": (_i, [_p]),
     "amgb_comm_unique_id_bytes": (_i, []),
     "amgb_comm_get_unique_id": (_i, [_p]),
     "amgb_comm_create": (_i, [_p, _i, _i, C.POINTER(_p)]),
@@ -271,6 +277,31 @@ class LinearInterpolator:
         out = np.empty(R.rows)
         _check(lib().amgb_csc_spmv(R.rows, R.cols, R.colptr, R.rowidx, R.val, _f64(v), out))
         return out
+
+
+class BilinearInterpolator2D(LinearInterpolator):
+    """Bilinear interpolation on an m x m grid of DOFs numbered k = y*m + x (TRANSFER_BILINEAR_2D):
+    P = P1 (x) P1 with LinearInterpolator's 1-D pattern P1, m_H = m_h // 2 lines, R = P^T.  No
+    reference counterpart: the 2-D coarsening that makes the V-cycle converge independently of the
+    grid size on 2-D problems, where the reference's 1-D rule semi-coarsens the flattened vector."""
+
+    transfer = TRANSFER_BILINEAR_2D
+
+    @staticmethod
+    def coarse_lines(m_h):
+        return lib().amgb_bilinear_coarse_lines(m_h)
+
+    def make_operators(self, n_h, n_H, level):
+        m_h, m_H = int(round(n_h ** 0.5)), int(round(n_H ** 0.5))
+        if m_h * m_h != n_h or m_H * m_H != n_H or m_H != self.coarse_lines(m_h):
+            raise InvalidArgument(EINVAL, "BilinearInterpolator2D: %d -> %d DOFs are not m^2 -> (m // 2)^2"
+                                  % (n_h, n_H))
+        nnz = lib().amgb_bilinear_nnz(m_h, m_H)
+        Pc, Pr, Pv = np.empty(n_H + 1, np.int32), np.empty(nnz, np.int32), np.empty(nnz)
+        Rc, Rr, Rv = np.empty(n_h + 1, np.int32), np.empty(nnz, np.int32), np.empty(nnz)
+        _check(lib().amgb_bilinear_make_operators(m_h, m_H, Pc, Pr, Pv, Rc, Rr, Rv))
+        self._P[level] = CscMatrix(n_h, n_H, Pc, Pr, Pv)
+        self._R[level] = CscMatrix(n_H, n_h, Rc, Rr, Rv)
 
 
 class DeviceMatrix:
@@ -501,6 +532,7 @@ class Multigrid:
         if fuse is not None:
             o.fuse = int(fuse)
         o.arith = int(arith)
+        o.transfer = int(getattr(interpolator, "transfer", TRANSFER_LINEAR))
         b = _f64(b)
         h = _p()
         if comm is None:
@@ -527,6 +559,10 @@ class Multigrid:
     # ---- reference getters (multigrid.hpp:339-354) ----
     def get_n_dofs(self, level):
         return lib().amgb_hierarchy_n_dofs(self.h, level)
+
+    def transfer(self):
+        """TRANSFER_* the hierarchy was built with."""
+        return lib().amgb_hierarchy_transfer(self.h)
 
     def get_tolerance(self):
         return lib().amgb_hierarchy_tolerance(self.h)

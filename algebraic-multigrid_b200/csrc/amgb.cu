@@ -19,6 +19,7 @@
 #include "host_setup.hpp"
 #include "fused_leg.cuh"
 #include "galerkin_dia.cuh"
+#include "galerkin_dia2d.cuh"
 #include "gs_wave.cuh"
 #include "kernels.cuh"
 #include "mid_levels.cuh"
@@ -40,6 +41,13 @@ __global__ void __launch_bounds__(256) k_galerkin_dia(gal::FineDia A, int n_c, i
                                                       double* __restrict__ val_c, int ld_c) {
   const int I = blockIdx.x * blockDim.x + threadIdx.x;
   if (I < n_c) gal::coarse_row(A, n_c, nd_c, off_c.v, I, val_c + I, ld_c);
+}
+
+// the same for the bilinear transfer of a 2-D hierarchy (galerkin_dia2d.cuh)
+__global__ void __launch_bounds__(256) k_galerkin_dia2d(gal::FineDia A, int m_h, int m_H, int nd_c, CoarseOffsets off_c,
+                                                        double* __restrict__ val_c, int ld_c) {
+  const int I = blockIdx.x * blockDim.x + threadIdx.x;
+  if (I < m_H * m_H) gal::coarse_row_2d(A, m_h, m_H, nd_c, off_c.v, I, val_c + I, ld_c);
 }
 
 thread_local std::string g_err;
@@ -718,6 +726,17 @@ struct Operator {
                n_coarse);
     });
   }
+  // bilinear transfer of a 2-D hierarchy: this operator is the m_h x m_h grid level, the coarse one m_H x m_H
+  void residual_restrict2d(const double* u, const double* f, int m_h, double* f_coarse, double* u_coarse, int m_H,
+                           cudaStream_t s) const {
+    if (m_H < 1) return;
+    with_view(rows_of_A(), [&](auto V) {
+      auto kern = dev::k_residual_restrict2d<decltype(V)>;
+      V.n_rows = n_mat;
+      LAUNCH(kern, dim3(blocks_for(m_H, dev::kRR2X), blocks_for(m_H, dev::kRR2Y)), 256, 0, s, V, u, f, m_h, f_coarse,
+             u_coarse, m_H);
+    });
+  }
   int rss_blocks() const { return std::max(1, blocks_for(n, 256)); }
   // partial must hold rss_blocks() doubles; out one double
   void rss(const double* u, const double* b, double* partial, double* out, cudaStream_t s) const {
@@ -752,6 +771,7 @@ void options_default(amgb_options* o) {
   if (const char* c = std::getenv("AMGB_COMPRESS"))
     if (std::string(c) == "1") o->fuse |= 64 | 128;
   o->arith = AMGB_ARITH_REFERENCE;
+  o->transfer = AMGB_TRANSFER_LINEAR;
   // the C++ mirror of the reference's headers has no argument for it: AMGB_ARITH=fast selects the fast
   // arithmetic for hierarchies created with the default options
   if (const char* a = std::getenv("AMGB_ARITH"))
@@ -810,6 +830,8 @@ struct amgb_hierarchy {
   amgb_options opt{};
   int L = 0;
   std::vector<int64_t> n;
+  std::vector<int64_t> m;  // grid lines per level of a 2-D hierarchy (n[l] = m[l]^2), empty otherwise
+  bool bilinear() const { return opt.transfer == AMGB_TRANSFER_BILINEAR_2D; }
   std::vector<std::unique_ptr<Operator>> ops;
   std::vector<LevelState> lv;
   DevBuf<double> partial, scalar;
@@ -1256,6 +1278,10 @@ struct amgb_hierarchy {
   void residual_restrict(int l, cudaStream_t s) {
     LevelState& F = lv[l];
     LevelState& C = lv[l + 1];
+    if (bilinear()) {  // (never sharded)
+      ops[l]->residual_restrict2d(F.u.p, F.f.p, (int)m[l], C.f.p, C.u.p, (int)m[l + 1], s);
+      return;
+    }
     if (!F.sharded) {
       ops[l]->residual_restrict(F.u.p, F.f.p, C.f.p, C.u.p, (int)n[l + 1], s);
       return;
@@ -1277,6 +1303,10 @@ struct amgb_hierarchy {
   void prolong_add(int l, cudaStream_t s) {
     LevelState& F = lv[l];
     LevelState& C = lv[l + 1];
+    if (bilinear()) {
+      prolong_add2d(C.u.p, F.u.p, l, s);
+      return;
+    }
     if (C.sharded) exchange(l + 1, C.u.p, s);  // needs e[s_c - 1]
     const int e_first = C.sharded ? (int)(C.s - C.halo_lo) : 0;
     if ((reinterpret_cast<uintptr_t>(F.u_own()) & 15) == 0 && (F.s & 1) == 0)
@@ -1285,6 +1315,22 @@ struct amgb_hierarchy {
     else
       LAUNCH(dev::k_prolong_add, blocks_for(F.n_own, 256), 256, 0, s, C.u.p, e_first, (int)n[l + 1],
              F.u_own(), (int)F.s, F.n_own);
+  }
+  // u_l += P_l e on a 2-D hierarchy (e: m_{l+1}^2 coarse values, u: m_l^2 fine values)
+  void prolong_add2d(const double* e, double* u, int l, cudaStream_t s) const {
+    if (m[l] < 1) return;
+    LAUNCH(dev::k_prolong_add2d, dim3(blocks_for(m[l], 256), (unsigned)blocks_for(m[l], 2)), 256, 0, s, e, (int)m[l + 1], u,
+           (int)m[l]);
+  }
+  // f_c = R_l r on a 2-D hierarchy
+  void restrict2d(const double* r, double* f_c, int l, cudaStream_t s) const {
+    if (m[l + 1] < 1) return;
+    LAUNCH(dev::k_restrict2d, dim3(blocks_for(m[l + 1], 256), (unsigned)m[l + 1]), 256, 0, s, r, (int)m[l], f_c,
+           (int)m[l + 1]);
+  }
+  // P_l of this hierarchy's transfer kind (host setup)
+  Csc prolongation(int l) const {
+    return bilinear() ? make_prolongation_2d(m[l], m[l + 1]) : make_prolongation(n[l], n[l + 1]);
   }
   void coarse_solve(cudaStream_t s) {  // multigrid.hpp:287-288
     const int nc = factor.n, bw = factor.bw;
@@ -1996,7 +2042,7 @@ struct amgb_hierarchy {
     }
     while ((int)host_mats.size() <= level) {  // multigrid.hpp:211-223
       const int l = (int)host_mats.size();
-      Csc P = make_prolongation(n[l - 1], n[l]);
+      Csc P = prolongation(l - 1);
       Csc R = transpose(P);
       host_mats.push_back(galerkin(R, host_mats[l - 1], P));
     }
@@ -2121,6 +2167,26 @@ int amgb_interp_make_operators(int64_t n_h, int64_t n_H, int* P_colptr, int* P_r
   });
 }
 
+int64_t amgb_bilinear_coarse_lines(int64_t m_h) { return m_h < 0 ? -1 : coarse_lines_2d(m_h); }
+int64_t amgb_bilinear_nnz(int64_t m_h, int64_t m_H) {
+  const int64_t k = amgb_interp_nnz(m_h, m_H);
+  return k < 0 ? -1 : k * k;
+}
+int amgb_bilinear_make_operators(int64_t m_h, int64_t m_H, int* P_colptr, int* P_rowidx, double* P_val,
+                                 int* R_colptr, int* R_rowidx, double* R_val) {
+  return guarded([&] {
+    if (m_h < 0 || m_H < 0) throw std::invalid_argument("negative size");
+    if (!P_colptr || !P_rowidx || !P_val || !R_colptr || !R_rowidx || !R_val) throw std::invalid_argument("null argument");
+    const Csc P = make_prolongation_2d(m_h, m_H);
+    const Csc R = transpose(P);
+    std::memcpy(P_colptr, P.colptr.data(), P.colptr.size() * sizeof(int));
+    std::memcpy(P_rowidx, P.rowidx.data(), P.rowidx.size() * sizeof(int));
+    std::memcpy(P_val, P.val.data(), P.val.size() * sizeof(double));
+    std::memcpy(R_colptr, R.colptr.data(), R.colptr.size() * sizeof(int));
+    std::memcpy(R_rowidx, R.rowidx.data(), R.rowidx.size() * sizeof(int));
+    std::memcpy(R_val, R.val.data(), R.val.size() * sizeof(double));
+  });
+}
 int amgb_linear_restrict(int64_t n_h, int64_t n_H, const double* r, double* out) {
   return guarded([&] {
     if (!r || !out || n_h < 0 || n_H < 0) throw std::invalid_argument("bad transfer arguments");
@@ -2479,6 +2545,22 @@ static bool device_build_levels(amgb_hierarchy* h, int n_rows, const int* colptr
   const int L = h->L;
   const int64_t nnz = colptr[n_rows];
   if (n_rows < 1 || nnz < 1) return false;
+  if (h->bilinear()) {
+    // the row-wise 2-D product needs a 3 x 3 grid stencil (every level below is one then); anything
+    // else is left to the host product
+    // entry (r, c) couples grid point c = (y, x) to r = c + d: allowed are d = dy m + dx with dy, dx in
+    // {-1, 0, 1} and x + dx inside the line (no entry across a line end); x is tracked, not divided out
+    const int m = (int)h->m[0];
+    if (m < 3) return false;
+    for (int c = 0, x = 0; c < n_rows; ++c, x = (x + 1 == m) ? 0 : x + 1)
+      for (int p = colptr[c]; p < colptr[c + 1]; ++p) {
+        if (val[p] == 0.0) continue;
+        const int d = rowidx[p] - c;
+        const int dy = (d > 1) ? 1 : (d < -1 ? -1 : 0);
+        const int dx = d - dy * m;
+        if (dx < -1 || dx > 1 || x + dx < 0 || x + dx >= m) return false;
+      }
+  }
   h->raw_rows = n_rows;
   h->raw_colptr.upload(colptr, (size_t)n_rows + 1, s);
   h->raw_rowidx.upload(rowidx, (size_t)nnz, s);
@@ -2547,13 +2629,16 @@ static bool device_build_levels(amgb_hierarchy* h, int n_rows, const int* colptr
     for (int d = 0; d < A.nd; ++d) A.off[d] = Fd.off[d];
     A.val = Fd.val.p;
     CoarseOffsets oc{};
-    const int nd_c = gal::coarse_offsets(A.nd, A.off, oc.v);
+    const int nd_c = h->bilinear() ? gal::coarse_offsets_2d((int)h->m[l], oc.v) : gal::coarse_offsets(A.nd, A.off, oc.v);
     if (nd_c < 1) return false;
     const int ld_c = (n_c + 31) / 32 * 32;
     DevBuf<double> out;
     out.alloc((size_t)nd_c * ld_c);
     out.zero(s);
-    LAUNCH(k_galerkin_dia, blocks_for(n_c, 256), 256, 0, s, A, n_c, nd_c, oc, out.p, ld_c);
+    if (h->bilinear())
+      LAUNCH(k_galerkin_dia2d, blocks_for(n_c, 256), 256, 0, s, A, (int)h->m[l - 1], (int)h->m[l], nd_c, oc, out.p, ld_c);
+    else
+      LAUNCH(k_galerkin_dia, blocks_for(n_c, 256), 256, 0, s, A, n_c, nd_c, oc, out.p, ld_c);
     std::vector<int> off_c(oc.v, oc.v + nd_c);
     if (!finalize_full_level(full[l], std::move(out), off_c, n_c, ld_c, s)) return false;
   }
@@ -2600,11 +2685,21 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
   if (n_rows != n_cols) throw std::invalid_argument("A must be square");
   if (o.smoother < 0 || o.smoother > 2) throw std::invalid_argument("unknown smoother kind");
   if (o.arith != AMGB_ARITH_REFERENCE && o.arith != AMGB_ARITH_FAST) throw std::invalid_argument("unknown arithmetic mode");
+  if (o.transfer != AMGB_TRANSFER_LINEAR && o.transfer != AMGB_TRANSFER_BILINEAR_2D)
+    throw std::invalid_argument("unknown transfer kind");
+  if (o.transfer == AMGB_TRANSFER_BILINEAR_2D) {
+    if (grid_lines(n_rows) < 1)
+      throw std::invalid_argument("the bilinear 2-D transfer needs an m x m grid operator, got " + std::to_string(n_rows) +
+                                  " rows (not a square number)");
+  }
   if (!b || !rowidx || !val) throw std::invalid_argument("null argument");
   require_device();
 
   std::unique_ptr<amgb_hierarchy> h(new amgb_hierarchy());
   h->opt = o;
+  // fuse bits 1-7 (folded prolongation, fused legs, coarse tail, mid levels, compressed formats) hard-code
+  // the 1-D transfer; a 2-D hierarchy runs the per-operator cycle with the zero-guess first sweep only
+  if (h->bilinear()) h->opt.fuse &= 1;
   h->L = o.n_levels;
   h->comm = comm;
   CUDA_CHECK(cudaGetDevice(&h->device));
@@ -2616,8 +2711,14 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
   // ---- level sizes (multigrid.hpp:127-130, :213-215) ----
   h->n.resize(L);
   h->n[0] = n_rows;
+  if (h->bilinear()) h->m.assign(1, grid_lines(n_rows));
   for (int l = 1; l < L; ++l) {
-    h->n[l] = coarse_dofs(h->n[l - 1]);
+    if (h->bilinear()) {
+      h->m.push_back(coarse_lines_2d(h->m[l - 1]));
+      h->n[l] = h->m[l] * h->m[l];
+    } else {
+      h->n[l] = coarse_dofs(h->n[l - 1]);
+    }
     if (h->n[l] < 1) throw std::invalid_argument("too many levels: level " + std::to_string(l) + " is empty");
   }
 
@@ -2639,7 +2740,7 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
     mats.resize(L);
     mats[0] = csc_from_arrays(n_rows, n_cols, colptr, rowidx, val);
     for (int l = 1; l < L; ++l) {
-      Csc P = make_prolongation(h->n[l - 1], h->n[l]);
+      Csc P = h->prolongation(l - 1);
       Csc R = transpose(P);
       mats[l] = galerkin(R, mats[l - 1], P);
     }
@@ -2803,6 +2904,8 @@ int amgb_hierarchy_create_sharded(amgb_comm* comm, int64_t min_rows_per_rank, in
                                   int64_t b_rows, const amgb_options* opt_in, amgb_hierarchy** out) {
   return guarded([&] {
     if (!comm) throw std::invalid_argument("null communicator");
+    if (opt_in && opt_in->transfer == AMGB_TRANSFER_BILINEAR_2D)
+      throw std::invalid_argument("the bilinear 2-D transfer is a single-GPU path (no sharded hierarchy)");
     CUDA_CHECK(cudaSetDevice(comm->device));
     create_hierarchy(comm, std::max<int64_t>(min_rows_per_rank, 1), n_rows, n_cols, colptr, rowidx, val, b,
                      b_rows, opt_in, out);
@@ -2907,6 +3010,7 @@ int amgb_hierarchy_set_stream(amgb_hierarchy* h, void* cuda_stream) {
   });
 }
 int amgb_hierarchy_n_levels(const amgb_hierarchy* h) { return h ? h->L : 0; }
+int amgb_hierarchy_transfer(const amgb_hierarchy* h) { return h ? h->opt.transfer : -1; }
 int64_t amgb_hierarchy_n_dofs(const amgb_hierarchy* h, int level) {
   return (h && level >= 0 && level < h->L) ? h->n[level] : -1;
 }
@@ -3165,8 +3269,11 @@ int amgb_restrict(amgb_hierarchy* h, int level, const double* r_fine, double* f_
     DevBuf<double> r, fc;
     r.upload(r_fine, h->n[level], h->stream);
     fc.alloc(h->n[level + 1]);
-    LAUNCH(dev::k_restrict, blocks_for(h->n[level + 1], 256), 256, 0, h->stream, r.p, (int)h->n[level],
-           fc.p, (int)h->n[level + 1]);
+    if (h->bilinear())
+      h->restrict2d(r.p, fc.p, level, h->stream);
+    else
+      LAUNCH(dev::k_restrict, blocks_for(h->n[level + 1], 256), 256, 0, h->stream, r.p, (int)h->n[level],
+             fc.p, (int)h->n[level + 1]);
     fc.download(f_coarse, h->stream);
     CUDA_CHECK(cudaStreamSynchronize(h->stream));
   });
@@ -3180,8 +3287,11 @@ int amgb_prolong_add(amgb_hierarchy* h, int level, const double* e_coarse, doubl
     DevBuf<double> e, uf;
     e.upload(e_coarse, h->n[level + 1], h->stream);
     uf.upload(u_fine, h->n[level], h->stream);
-    LAUNCH(dev::k_prolong_add, blocks_for(h->n[level], 256), 256, 0, h->stream, e.p, 0, (int)h->n[level + 1],
-           uf.p, 0, (int)h->n[level]);
+    if (h->bilinear())
+      h->prolong_add2d(e.p, uf.p, level, h->stream);
+    else
+      LAUNCH(dev::k_prolong_add, blocks_for(h->n[level], 256), 256, 0, h->stream, e.p, 0, (int)h->n[level + 1],
+             uf.p, 0, (int)h->n[level]);
     uf.download(u_fine, h->stream);
     CUDA_CHECK(cudaStreamSynchronize(h->stream));
   });
@@ -3300,7 +3410,8 @@ int amgb_hierarchy_galerkin_device(amgb_hierarchy* h, int level, double* ms_out,
     for (int d = 0; d < A.nd; ++d) A.off[d] = F.dia.off[d];
     A.val = F.dia.val.p;
     CoarseOffsets oc{};
-    const int nd_c = gal::coarse_offsets(A.nd, A.off, oc.v);
+    const bool bl = h->bilinear();
+    const int nd_c = bl ? gal::coarse_offsets_2d((int)h->m[level + 1], oc.v) : gal::coarse_offsets(A.nd, A.off, oc.v);
     if (nd_c < 0) throw ApiError(AMGB_ESTATE, "coarse operator has too many diagonals");
     const int n_c = (int)h->n[level + 1];
     const int ld_c = (n_c + 31) / 32 * 32;
@@ -3310,9 +3421,16 @@ int amgb_hierarchy_galerkin_device(amgb_hierarchy* h, int level, double* ms_out,
     cudaEvent_t e0, e1;
     CUDA_CHECK(cudaEventCreate(&e0));
     CUDA_CHECK(cudaEventCreate(&e1));
-    LAUNCH(k_galerkin_dia, blocks_for(n_c, 256), 256, 0, h->stream, A, n_c, nd_c, oc, out.p, ld_c);  // warm-up
+    auto once = [&] {
+      if (bl)
+        LAUNCH(k_galerkin_dia2d, blocks_for(n_c, 256), 256, 0, h->stream, A, (int)h->m[level], (int)h->m[level + 1], nd_c,
+               oc, out.p, ld_c);
+      else
+        LAUNCH(k_galerkin_dia, blocks_for(n_c, 256), 256, 0, h->stream, A, n_c, nd_c, oc, out.p, ld_c);
+    };
+    once();  // warm-up
     CUDA_CHECK(cudaEventRecord(e0, h->stream));
-    LAUNCH(k_galerkin_dia, blocks_for(n_c, 256), 256, 0, h->stream, A, n_c, nd_c, oc, out.p, ld_c);
+    once();
     CUDA_CHECK(cudaEventRecord(e1, h->stream));
     CUDA_CHECK(cudaEventSynchronize(e1));
     float ms = 0.f;
@@ -3574,11 +3692,17 @@ int amgb_time_kernel(amgb_hierarchy* h, int level, int kind, int warmup, int rep
           A.residual(su, S.f.p, S.tmp_own(), s);
           break;
         case 2:
-          A.residual_restrict(scratch_u.p, S.f.p, scratch_c2.p, scratch_c.p, (int)h->n[level + 1], s);
+          if (h->bilinear())
+            A.residual_restrict2d(scratch_u.p, S.f.p, (int)h->m[level], scratch_c2.p, scratch_c.p, (int)h->m[level + 1], s);
+          else
+            A.residual_restrict(scratch_u.p, S.f.p, scratch_c2.p, scratch_c.p, (int)h->n[level + 1], s);
           break;
         case 3:
-          LAUNCH(dev::k_prolong_add2, blocks_for((h->n[level] + 1) / 2, 256), 256, 0, s, scratch_c.p, 0,
-                 (int)h->n[level + 1], scratch_u.p, 0, (int)h->n[level]);
+          if (h->bilinear())
+            h->prolong_add2d(scratch_c.p, scratch_u.p, level, s);
+          else
+            LAUNCH(dev::k_prolong_add2, blocks_for((h->n[level] + 1) / 2, 256), 256, 0, s, scratch_c.p, 0,
+                   (int)h->n[level + 1], scratch_u.p, 0, (int)h->n[level]);
           break;
         default:
           throw std::invalid_argument("unknown kernel kind");

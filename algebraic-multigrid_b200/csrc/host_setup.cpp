@@ -136,6 +136,41 @@ Csc make_prolongation(int64_t n_h, int64_t n_H) {
   return P;
 }
 
+int64_t coarse_lines_2d(int64_t m_h) { return m_h / 2; }
+
+Csc make_prolongation_2d(int64_t m_h, int64_t m_H) {
+  const Csc P1 = make_prolongation(m_h, m_H);
+  const int64_t rows = m_h * m_h, cols = m_H * m_H;
+  if (rows > std::numeric_limits<int>::max() || 9 * cols > std::numeric_limits<int>::max())
+    throw std::overflow_error("make_prolongation_2d: exceeds int32 indexing");
+  Csc P;
+  P.rows = static_cast<int>(rows);
+  P.cols = static_cast<int>(cols);
+  P.colptr.resize(cols + 1);
+  P.rowidx.reserve(9 * cols);
+  P.val.reserve(9 * cols);
+  // column (Y, X): rows (y, x) for y in column Y of P1, x in column X of P1, y-major = ascending row
+  for (int64_t Y = 0; Y < m_H; ++Y)
+    for (int64_t X = 0; X < m_H; ++X) {
+      P.colptr[Y * m_H + X] = static_cast<int>(P.rowidx.size());
+      for (int p = P1.colptr[Y]; p < P1.colptr[Y + 1]; ++p)
+        for (int q = P1.colptr[X]; q < P1.colptr[X + 1]; ++q) {
+          P.rowidx.push_back(static_cast<int>(P1.rowidx[p] * m_h + P1.rowidx[q]));
+          P.val.push_back(P1.val[p] * P1.val[q]);
+        }
+    }
+  P.colptr[cols] = static_cast<int>(P.rowidx.size());
+  return P;
+}
+
+int64_t grid_lines(int64_t n) {
+  if (n < 0) return -1;
+  int64_t m = static_cast<int64_t>(std::llround(std::sqrt(static_cast<double>(n))));
+  while (m > 0 && m * m > n) --m;
+  while ((m + 1) * (m + 1) <= n) ++m;
+  return m * m == n ? m : -1;
+}
+
 Csc multiply(const Csc& L, const Csc& R) {
   if (L.cols != R.rows) throw std::invalid_argument("multiply: inner dimensions differ");
   Csc C;

@@ -37,6 +37,13 @@ void grid_rhs(int64_t n, double* b);
 // ---- interpolation + Galerkin ----
 int64_t coarse_dofs(int64_t fine_dofs);
 Csc make_prolongation(int64_t n_h, int64_t n_H);
+// Bilinear transfer on an m x m grid (DOF k = y*m + x): m_H = m_h / 2 lines per coarse level, so
+// every fine line is covered by some coarse line also when m_h is even; P = P1 (x) P1 with P1 =
+// make_prolongation(m_h, m_H), columns in ascending coarse index, rows ascending inside a column.
+int64_t coarse_lines_2d(int64_t m_h);
+Csc make_prolongation_2d(int64_t m_h, int64_t m_H);
+// m with m * m == n, or -1
+int64_t grid_lines(int64_t n);
 // Eigen 3.4.0 conservative ColMajor product: entry (i,j) = sum over ascending k
 // of L(i,k)*R(k,j); numerical zeros kept; result columns sorted.
 Csc multiply(const Csc& L, const Csc& R);

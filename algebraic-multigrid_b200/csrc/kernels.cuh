@@ -597,6 +597,116 @@ __global__ void __launch_bounds__(256) k_prolong_add(const double* __restrict__ 
   u[t] = __dadd_rn(u[t], prolong_at(e, e_first, n_coarse, fine_first + t));
 }
 
+// ------------------------------------------------------------------ bilinear transfer (2-D grids)
+// AMGB_TRANSFER_BILINEAR_2D on an m_h x m_h grid (DOF k = y*m_h + x), m_H = m_h / 2: coarse point
+// (Y, X) restricts from / prolongs to the fine points (2Y + a, 2X + b), a, b in {0, 1, 2}, inside the
+// grid, with weight w(a) * w(b), w = (.5, 1, .5) (P = P1 (x) P1, R = P^T).  Sums run over ascending
+// column index from +0, as Eigen's sparse x dense product (the oracle's spmv) does; every weight is a
+// power of two, so the products are exact and the result is bit-identical in both arithmetic modes.
+__device__ __forceinline__ double bl_w(int a) { return a == 1 ? 1.0 : 0.5; }
+
+// stand-alone restriction f_c = R r, one thread per coarse point
+__global__ void __launch_bounds__(256) k_restrict2d(const double* __restrict__ r, int m_h,
+                                                    double* __restrict__ f_coarse, int m_H) {
+  const int X = blockIdx.x * blockDim.x + threadIdx.x, Y = blockIdx.y;
+  if (X >= m_H) return;
+  double acc = 0.0;
+#pragma unroll
+  for (int a = 0; a < 3; ++a) {
+    const int y = 2 * Y + a;
+    if (y >= m_h) break;
+#pragma unroll
+    for (int b = 0; b < 3; ++b) {
+      const int x = 2 * X + b;
+      if (x >= m_h) break;
+      acc = __dadd_rn(acc, __dmul_rn(bl_w(a) * bl_w(b), r[(size_t)y * m_h + x]));
+    }
+  }
+  f_coarse[(size_t)Y * m_H + X] = acc;
+}
+
+// Fused residual + restriction: f_c = R (f - A u), u_c = 0 (multigrid.hpp:272-282).  A block owns a
+// tile of kRR2Y x kRR2X coarse points; it forms the residuals of the (2 kRR2Y + 1) x (2 kRR2X + 1)
+// fine points under the tile in shared memory (k_residual's per-row arithmetic) and restricts from
+// there, so r never reaches HBM.  Neighbouring tiles share one fine line / column: 17 x 129 residuals
+// for 16 x 128 distinct ones, 7 % formed twice.
+constexpr int kRR2X = 64, kRR2Y = 8;
+template <class M>
+__global__ void __launch_bounds__(256) k_residual_restrict2d(M A, const double* __restrict__ u,
+                                                             const double* __restrict__ f, int m_h,
+                                                             double* __restrict__ f_coarse,
+                                                             double* __restrict__ u_coarse, int m_H) {
+  constexpr int FX = 2 * kRR2X + 1, FY = 2 * kRR2Y + 1;
+  __shared__ double r[FY * FX];
+  const int X0 = blockIdx.x * kRR2X, Y0 = blockIdx.y * kRR2Y;
+  const int x0 = 2 * X0, y0 = 2 * Y0;
+  for (int p = threadIdx.x; p < FY * FX; p += blockDim.x) {
+    const int fy = p / FX, fx = p - fy * FX;
+    const int y = y0 + fy, x = x0 + fx;
+    double v = 0.0;
+    if (y < m_h && x < m_h) {
+      const int row = y * m_h + x;
+      v = row_residual(A, row, row, u, f[row]);
+    }
+    r[p] = v;
+  }
+  __syncthreads();
+  for (int p = threadIdx.x; p < kRR2Y * kRR2X; p += blockDim.x) {
+    const int ty = p / kRR2X, tx = p - ty * kRR2X;
+    const int Y = Y0 + ty, X = X0 + tx;
+    if (Y >= m_H || X >= m_H) continue;
+    double acc = 0.0;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+      if (2 * Y + a >= m_h) break;
+#pragma unroll
+      for (int b = 0; b < 3; ++b) {
+        if (2 * X + b >= m_h) break;
+        acc = __dadd_rn(acc, __dmul_rn(bl_w(a) * bl_w(b), r[(2 * ty + a) * FX + 2 * tx + b]));
+      }
+    }
+    const size_t J = (size_t)Y * m_H + X;
+    f_coarse[J] = acc;
+    if (u_coarse) u_coarse[J] = 0.0;
+  }
+}
+
+// (P e) at fine point (y, x): fine coordinate y takes coarse Y = (y - 1) / 2 with weight 1 when odd, and
+// Y = y / 2 - 1, y / 2 (those inside the coarse grid) with weight .5 each when even; the terms are summed
+// in ascending coarse index (Y-major).  Fully unrolled and predicated, so all loads are independent.
+__device__ __forceinline__ double prolong2d_at(const double* __restrict__ e, int m_H, int y, int x) {
+  const int ylo = (y & 1) ? (y >> 1) : max((y >> 1) - 1, 0), yhi = (y & 1) ? (y >> 1) : min(y >> 1, m_H - 1);
+  const int xlo = (x & 1) ? (x >> 1) : max((x >> 1) - 1, 0), xhi = (x & 1) ? (x >> 1) : min(x >> 1, m_H - 1);
+  const double w = ((y & 1) ? 1.0 : 0.5) * ((x & 1) ? 1.0 : 0.5);
+  double v[4];
+#pragma unroll
+  for (int i = 0; i < 2; ++i)
+#pragma unroll
+    for (int j = 0; j < 2; ++j)
+      v[2 * i + j] = (ylo + i <= yhi && xlo + j <= xhi) ? e[(size_t)(ylo + i) * m_H + xlo + j] : 0.0;
+  double acc = 0.0;
+#pragma unroll
+  for (int i = 0; i < 2; ++i)
+#pragma unroll
+    for (int j = 0; j < 2; ++j)
+      if (ylo + i <= yhi && xlo + j <= xhi) acc = __dadd_rn(acc, __dmul_rn(w, v[2 * i + j]));
+  return acc;
+}
+
+// u += P e: a thread owns fine column x of the two fine lines 2 blockIdx.y, 2 blockIdx.y + 1 (an even and
+// an odd line, which share their coarse lines), with every load issued before the first add.
+__global__ void __launch_bounds__(256) k_prolong_add2d(const double* __restrict__ e, int m_H,
+                                                       double* __restrict__ u, int m_h) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = 2 * blockIdx.y;
+  if (x >= m_h) return;
+  const bool two = y + 1 < m_h;
+  const size_t k = (size_t)y * m_h + x;
+  const double u0 = u[k], u1 = two ? u[k + m_h] : 0.0;
+  const double a0 = prolong2d_at(e, m_H, y, x), a1 = two ? prolong2d_at(e, m_H, y + 1, x) : 0.0;
+  u[k] = __dadd_rn(u0, a0);
+  if (two) u[k + m_h] = __dadd_rn(u1, a1);
+}
+
 // ------------------------------------------------------------------ peer-memory halo exchange
 // One launch per exchange site (the stand-alone exchange of the per-operator sharded path and of
 // the out-of-cycle sites; the fused legs push their boundary rows themselves, stream_leg.cuh).

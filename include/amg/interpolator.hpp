@@ -77,9 +77,11 @@ class InterpolatorBase {
   virtual ~InterpolatorBase() {}
 
   virtual void make_operators(size_t n_h_dofs, size_t n_H_dofs, size_t level) = 0;
-  // true when P is the reference's linear interpolation, which the device kernels apply
-  // matrix-free; other interpolators are not supported by the GPU driver
-  virtual bool is_linear_interpolation() const { return false; }
+  // AMGB_TRANSFER_* of the device kernels that apply this interpolator's operators matrix-free
+  // (-1: none, the GPU driver cannot run it)
+  virtual int device_transfer() const { return -1; }
+  // true when P is the reference's linear interpolation
+  bool is_linear_interpolation() const { return device_transfer() == AMGB_TRANSFER_LINEAR; }
 
   // :52-56 and :64-68 -- get_P(level) * v and get_R(level) * v with the operators that are
   // STORED, whoever put them there (make_operators of any subclass, set_level_to_P/R).  When the
@@ -135,7 +137,47 @@ class LinearInterpolator : public InterpolatorBase<EleType> {
     this->set_level_to_P(level, P);
     this->set_level_to_R(level, R);
   }
-  bool is_linear_interpolation() const override { return true; }
+  int device_transfer() const override { return AMGB_TRANSFER_LINEAR; }
+};
+
+// Bilinear interpolation on an m x m grid of DOFs numbered k = y*m + x (no reference counterpart):
+// P = P1 (x) P1 with LinearInterpolator's 1-D pattern P1, m_H = m_h / 2, R = P^T.  The 2-D
+// coarsening under which the V-cycle converges independently of the grid size on 2-D problems.
+template <class EleType>
+class BilinearInterpolator2D : public InterpolatorBase<EleType> {
+ public:
+  using InterpolatorBase<EleType>::InterpolatorBase;
+
+  void make_operators(size_t n_h_dofs, size_t n_H_dofs, size_t level) override {
+    const int64_t m_h = lines(n_h_dofs), m_H = lines(n_H_dofs);
+    if (m_h < 0 || m_H < 0 || m_H != amgb_bilinear_coarse_lines(m_h))
+      throw std::invalid_argument("BilinearInterpolator2D: " + std::to_string(n_h_dofs) + " -> " +
+                                  std::to_string(n_H_dofs) + " DOFs are not m^2 -> (m / 2)^2");
+    const int64_t nnz = amgb_bilinear_nnz(m_h, m_H);
+    std::vector<int> Pc(n_H_dofs + 1), Pr(nnz), Rc(n_h_dofs + 1), Rr(nnz);
+    std::vector<double> Pv(nnz), Rv(nnz);
+    detail::check(amgb_bilinear_make_operators(m_h, m_H, Pc.data(), Pr.data(), Pv.data(), Rc.data(), Rr.data(),
+                                               Rv.data()));
+#if AMGB_HAVE_EIGEN
+    SparseMatrixT<EleType> P = Eigen::Map<const Eigen::SparseMatrix<double>>(
+        (int)n_h_dofs, (int)n_H_dofs, nnz, Pc.data(), Pr.data(), Pv.data());
+    SparseMatrixT<EleType> R = Eigen::Map<const Eigen::SparseMatrix<double>>(
+        (int)n_H_dofs, (int)n_h_dofs, nnz, Rc.data(), Rr.data(), Rv.data());
+#else
+    SparseMatrixT<EleType> P((int)n_h_dofs, (int)n_H_dofs, std::move(Pc), std::move(Pr), std::move(Pv));
+    SparseMatrixT<EleType> R((int)n_H_dofs, (int)n_h_dofs, std::move(Rc), std::move(Rr), std::move(Rv));
+#endif
+    this->set_level_to_P(level, P);
+    this->set_level_to_R(level, R);
+  }
+  int device_transfer() const override { return AMGB_TRANSFER_BILINEAR_2D; }
+
+ private:
+  static int64_t lines(size_t n) {  // m with m * m == n, else -1
+    int64_t m = 0;
+    while ((m + 1) * (m + 1) <= (int64_t)n) ++m;
+    return m * m == (int64_t)n ? m : -1;
+  }
 };
 
 }  // namespace AMG

@@ -61,9 +61,11 @@ class Multigrid {
       if (!smoother || smoother->device_kind() < 0)
         throw std::invalid_argument("the GPU driver needs a SparseGaussSeidel, DampedJacobi or "
                                     "MulticolorGaussSeidel smoother");
-      if (!interpolator || !interpolator->is_linear_interpolation())
-        throw std::invalid_argument("the GPU driver applies LinearInterpolator's operators matrix-free");
+      if (!interpolator || interpolator->device_transfer() < 0)
+        throw std::invalid_argument("the GPU driver applies the operators of LinearInterpolator or "
+                                    "BilinearInterpolator2D matrix-free");
     }
+    if (interpolator && interpolator->device_transfer() >= 0) opt.transfer = interpolator->device_transfer();
     if (smoother && smoother->device_kind() >= 0) {
       opt.smoother = smoother->device_kind();
       opt.smoother_iters = (int64_t)smoother->n_iters;
