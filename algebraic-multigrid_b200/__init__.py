@@ -18,7 +18,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libamgb.so")
 
 OK, EINVAL, ECUDA, ENCCL, ESTATE = 0, 1, 2, 3, 4
-SMOOTHER_GS, SMOOTHER_JACOBI, SMOOTHER_COLOR_GS = 0, 1, 2
+SMOOTHER_GS, SMOOTHER_JACOBI, SMOOTHER_COLOR_GS, SMOOTHER_LINE_GS = 0, 1, 2, 3
+LINES_X, LINES_Y, LINES_ALTERNATING = 0, 1, 2
 GS_AUTO, GS_LEVELSCHED, GS_LINESCAN = 0, 1, 2
 GS_KERNEL_FRONTS, GS_KERNEL_LINESCAN, GS_KERNEL_WAVE = 0, 1, 2
 ARITH_REFERENCE, ARITH_FAST = 0, 1
@@ -35,7 +36,7 @@ class Options(C.Structure):
                 ("smoother", _i), ("smoother_iters", _l), ("omega", _d),
                 ("gs_mode", _i), ("use_graph", _i),
                 ("skip_dead_coarse_smooth", _i), ("fuse", _i), ("arith", _i),
-                ("transfer", _i)]
+                ("transfer", _i), ("lines", _i)]
 
 
 class AmgbError(RuntimeError):
@@ -75,6 +76,7 @@ SIGNATURES = {
     "amgb_smooth_gs": (_i, [_p, _pd, _pd, _d, _l, _l, _i, C.POINTER(_l), C.POINTER(_d)]),
     "amgb_smooth_jacobi": (_i, [_p, _pd, _pd, _d, _l]),
     "amgb_smooth_color_gs": (_i, [_p, _pd, _pd, _l]),
+    "amgb_smooth_line_gs": (_i, [_p, _pd, _pd, _l, _i]),
     "amgb_matrix_coloring": (_i, [_p, C.POINTER(_i), _pi]),
     "amgb_residual": (_i, [_p, _pd, _pd, _pd]),
     "amgb_rss": (_i, [_p, _pd, _pd, C.POINTER(_d)]),
@@ -474,6 +476,22 @@ class MulticolorGaussSeidel(SmootherBase):
         _check(lib().amgb_smooth_color_gs(_mirror(A).h, u, _f64(b), self.n_iters))
 
 
+class LineGaussSeidel(SmootherBase):
+    """Zebra line Gauss-Seidel on an m x m grid operator (include/amgb.h, AMGB_SMOOTHER_LINE_GS);
+    `lines` is LINES_X (strong x-coupling), LINES_Y or LINES_ALTERNATING.  Multigrid needs a
+    BilinearInterpolator2D with it."""
+    kind = SMOOTHER_LINE_GS
+
+    def __init__(self, n_iters=1, lines=LINES_X):
+        super().__init__(n_iters)
+        if lines not in (LINES_X, LINES_Y, LINES_ALTERNATING):
+            raise ValueError("`lines` must be LINES_X, LINES_Y or LINES_ALTERNATING, got %r" % (lines,))
+        self.lines = lines
+
+    def smooth(self, A, u, b):
+        _check(lib().amgb_smooth_line_gs(_mirror(A).h, u, _f64(b), self.n_iters, self.lines))
+
+
 class Comm:
     """One NCCL communicator per process (amgb_comm).  `exchange_id` is a callable that
     takes rank 0's id bytes (or None on other ranks) and returns rank 0's bytes on every
@@ -533,6 +551,7 @@ class Multigrid:
             o.fuse = int(fuse)
         o.arith = int(arith)
         o.transfer = int(getattr(interpolator, "transfer", TRANSFER_LINEAR))
+        o.lines = int(getattr(smoother, "lines", LINES_X))
         b = _f64(b)
         h = _p()
         if comm is None:

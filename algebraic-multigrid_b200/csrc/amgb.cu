@@ -22,6 +22,7 @@
 #include "galerkin_dia2d.cuh"
 #include "gs_wave.cuh"
 #include "kernels.cuh"
+#include "line_gs.cuh"
 #include "mid_levels.cuh"
 #include "setup_dia.cuh"
 #include "stream_leg_api.hpp"
@@ -610,6 +611,110 @@ struct Operator {
     LAUNCH(kern, 1, lines_T + 32, lines_smem, s, L, g, u);  // + the producer warp
   }
 
+  // Zebra line Gauss-Seidel (line_gs.cuh) on an m x m grid operator: per direction the factors
+  // [sub | den (or 1 / den) | cp], each n doubles in step-major order, built on first use
+  int lgs_m = 0;
+  lgs::Grid lgs_grid{};
+  DevBuf<double> lgs_fac[2];
+  // `what` names the operator in the messages ("level 3"); throws std::invalid_argument when the
+  // operator is not a 3 x 3 grid stencil or a line has a zero pivot
+  void ensure_line_gs(int m, int D, bool fast, const std::string& what, cudaStream_t s) {
+    if (lgs_fac[D].p) return;
+    if (!lgs_m) {
+      const DevMat& R = rows_of_A();
+      if (m < 3)
+        throw std::invalid_argument("line Gauss-Seidel needs at least 3 grid lines: " + what + " has " +
+                                    std::to_string(m));
+      const std::string no_grid = "line Gauss-Seidel: " + what + " is not an m x m grid operator with a 3 x 3 stencil "
+                                  "that never couples across the end of a line";
+      if (block || !R.is_dia || R.dia.rows.p || R.dia.n_rows != n || (int64_t)m * m != n)
+        throw std::invalid_argument(no_grid);
+      const DevDia& D9 = R.dia;
+      const gsw::Plan Pl = gsw::plan_for(D9.off, D9.n_diag, n, m);
+      if (!Pl.ok) throw std::invalid_argument(no_grid);
+      gsw::CheckArgs C{};
+      C.val = D9.val.p;
+      C.ld = D9.ld;
+      C.n_diag = D9.n_diag;
+      C.n = n;
+      C.m = m;
+      C.n_lines = m;
+      for (int d = 0; d < D9.n_diag; ++d) C.e_of[d] = Pl.e_of[d];
+      DevBuf<unsigned> flags;  // [0] slots in use, [1] "an entry leaves the grid"
+      flags.alloc(2);
+      flags.zero(s);
+      LAUNCH(gsw::k_gsw_check, blocks_for(n, 256), 256, 0, s, C, flags.p, reinterpret_cast<int*>(flags.p + 1));
+      unsigned got[2] = {0, 0};
+      CUDA_CHECK(cudaMemcpyAsync(got, flags.p, sizeof(got), cudaMemcpyDeviceToHost, s));
+      CUDA_CHECK(cudaStreamSynchronize(s));
+      if (got[1]) throw std::invalid_argument(no_grid);
+      lgs_grid.val = D9.val.p;
+      lgs_grid.ld = D9.ld;
+      lgs_grid.m = m;
+      for (int e = 0; e < gsw::kSlots; ++e) lgs_grid.d_of[e] = Pl.d_of[e];
+      lgs_m = m;
+    }
+    DevBuf<double> fac;
+    fac.alloc(3 * (size_t)n);
+    DevBuf<int> bad;
+    bad.alloc(1);
+    const int none = INT_MAX;
+    CUDA_CHECK(cudaMemcpyAsync(bad.p, &none, sizeof(int), cudaMemcpyHostToDevice, s));
+    auto kern = fast ? lgs::k_line_factor<true> : lgs::k_line_factor<false>;
+    LAUNCH(kern, blocks_for(m, 128), 128, 0, s, lgs_grid, D, fac.p, fac.p + n, fac.p + 2 * (size_t)n, bad.p);
+    int row = none;
+    CUDA_CHECK(cudaMemcpyAsync(&row, bad.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+    CUDA_CHECK(cudaStreamSynchronize(s));
+    if (row != none)
+      throw std::invalid_argument("line Gauss-Seidel: zero pivot in the " + std::string(D == lgs::kX ? "X" : "Y") +
+                                  "-line solve of " + what + " at row " + std::to_string(row));
+    lgs_fac[D] = std::move(fac);
+  }
+  // one pass: every line of direction D and colour c solved exactly (g: n scratch doubles)
+  template <int D>
+  void line_pass(int c, bool fast, const double* f, double* u, double* g, cudaStream_t s) const {
+    const int m = lgs_m, nl = lgs::lines_of_colour(m, c);
+    if (nl < 1) return;
+    const double* fac = lgs_fac[D].p;
+    if (fast) {
+      LAUNCH((lgs::k_line_rhs<D, true>), blocks_for((int64_t)nl * m, 256), 256, 0, s, lgs_grid, c, f, u, g);
+      LAUNCH((lgs::k_line_solve<D, true>), blocks_for(nl, lgs::kSolveThreads), lgs::kSolveThreads, 0, s, m, c, fac,
+             fac + n, fac + 2 * (size_t)n, g, u);
+    } else {
+      LAUNCH((lgs::k_line_rhs<D, false>), blocks_for((int64_t)nl * m, 256), 256, 0, s, lgs_grid, c, f, u, g);
+      LAUNCH((lgs::k_line_solve<D, false>), blocks_for(nl, lgs::kSolveThreads), lgs::kSolveThreads, 0, s, m, c, fac,
+             fac + n, fac + 2 * (size_t)n, g, u);
+    }
+  }
+  void line_pass(int D, int c, bool fast, const double* f, double* u, double* g, cudaStream_t s) const {
+    if (D == lgs::kX) line_pass<lgs::kX>(c, fast, f, u, g, s);
+    else line_pass<lgs::kY>(c, fast, f, u, g, s);
+  }
+  static int line_dirs(int lines, int* dirs) {
+    if (lines == AMGB_LINES_Y) {
+      dirs[0] = lgs::kY;
+      return 1;
+    }
+    dirs[0] = lgs::kX;
+    dirs[1] = lgs::kY;
+    return lines == AMGB_LINES_ALTERNATING ? 2 : 1;
+  }
+  void ensure_line_gs_lines(int m, int lines, bool fast, const std::string& what, cudaStream_t s) {
+    int dirs[2];
+    const int nd = line_dirs(lines, dirs);
+    for (int i = 0; i < nd; ++i) ensure_line_gs(m, dirs[i], fast, what, s);
+  }
+  // forward half: each direction in order, colour 0 then 1; backward half: reversed
+  void line_gs_half(bool forward, int lines, bool fast, const double* f, double* u, double* g, cudaStream_t s) const {
+    int dirs[2];
+    const int nd = line_dirs(lines, dirs);
+    for (int i = 0; i < nd; ++i) {
+      const int D = dirs[forward ? i : nd - 1 - i];
+      line_pass(D, forward ? 0 : 1, fast, f, u, g, s);
+      line_pass(D, forward ? 1 : 0, fast, f, u, g, s);
+    }
+  }
+
   // first owned global row of a row block (0 for a whole level); the colour mirrors list GLOBAL rows
   int block_row0 = 0;
   void ensure_colors(cudaStream_t s) {
@@ -772,6 +877,7 @@ void options_default(amgb_options* o) {
     if (std::string(c) == "1") o->fuse |= 64 | 128;
   o->arith = AMGB_ARITH_REFERENCE;
   o->transfer = AMGB_TRANSFER_LINEAR;
+  o->lines = AMGB_LINES_X;
   // the C++ mirror of the reference's headers has no argument for it: AMGB_ARITH=fast selects the fast
   // arithmetic for hierarchies created with the default options
   if (const char* a = std::getenv("AMGB_ARITH"))
@@ -1129,6 +1235,10 @@ struct amgb_hierarchy {
       if (!lv[l].tmp.p) lv[l].tmp.alloc(lv[l].n_vec() + 4);
     }
     if (opt.smoother == AMGB_SMOOTHER_COLOR_GS) ops[l]->ensure_colors(stream);
+    if (opt.smoother == AMGB_SMOOTHER_LINE_GS) {
+      ops[l]->ensure_line_gs_lines((int)m[l], opt.lines, fast_arith(), "level " + std::to_string(l), stream);
+      if (!lv[l].tmp.p) lv[l].tmp.alloc(lv[l].n_vec() + 4);
+    }
   }
 
   // Halo exchange of a halo-extended level vector with ranks g-1 / g+1: one grouped
@@ -1228,6 +1338,11 @@ struct amgb_hierarchy {
         for (int64_t it = 0; it < iters; ++it) {  // smoother.hpp:195-198
           A.gs_direction(true, S.f.p, S.u.p, S.tmp.p, opt.gs_mode, s);
           A.gs_direction(false, S.f.p, S.u.p, S.tmp.p, opt.gs_mode, s);
+        }
+      } else if (opt.smoother == AMGB_SMOOTHER_LINE_GS) {
+        for (int64_t it = 0; it < iters; ++it) {
+          A.line_gs_half(true, opt.lines, fast_arith(), S.f.p, S.u.p, S.tmp.p, s);
+          A.line_gs_half(false, opt.lines, fast_arith(), S.f.p, S.u.p, S.tmp.p, s);
         }
       } else if (opt.smoother == AMGB_SMOOTHER_COLOR_GS) {
         // Row-block sharded level: the colour mirrors list global rows, so the vectors are handed over
@@ -2330,6 +2445,26 @@ int amgb_smooth_color_gs(amgb_matrix* A, double* u, const double* b, int64_t n_i
     CUDA_CHECK(cudaStreamSynchronize(s));
   });
 }
+int amgb_smooth_line_gs(amgb_matrix* A, double* u, const double* b, int64_t n_iters, int lines) {
+  return guarded([&] {
+    if (!A || !u || !b) throw std::invalid_argument("null argument");
+    if (lines != AMGB_LINES_X && lines != AMGB_LINES_Y && lines != AMGB_LINES_ALTERNATING)
+      throw std::invalid_argument("unknown line direction setting " + std::to_string(lines));
+    const int m = (int)grid_lines(A->op.n);
+    if (m < 1) throw std::invalid_argument("line Gauss-Seidel needs an m x m grid operator (rows not a square number)");
+    CUDA_CHECK(cudaSetDevice(A->device));
+    cudaStream_t s = A->stream;
+    A->op.ensure_line_gs_lines(m, lines, false, "the matrix", s);
+    A->u.upload(u, A->op.n, s);
+    A->b.upload(b, A->op.n, s);
+    for (int64_t it = 0; it < n_iters; ++it) {
+      A->op.line_gs_half(true, lines, false, A->b.p, A->u.p, A->r.p, s);
+      A->op.line_gs_half(false, lines, false, A->b.p, A->u.p, A->r.p, s);
+    }
+    A->u.download(u, s);
+    CUDA_CHECK(cudaStreamSynchronize(s));
+  });
+}
 int amgb_matrix_coloring(amgb_matrix* A, int* n_colors, int* color) {
   return guarded([&] {
     if (!A) throw std::invalid_argument("null argument");
@@ -2683,7 +2818,7 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
                                 std::to_string(n_rows) + " and " + std::to_string(b_rows));
   if (o.n_levels < 1) throw std::invalid_argument("n_levels must be >= 1");
   if (n_rows != n_cols) throw std::invalid_argument("A must be square");
-  if (o.smoother < 0 || o.smoother > 2) throw std::invalid_argument("unknown smoother kind");
+  if (o.smoother < 0 || o.smoother > 3) throw std::invalid_argument("unknown smoother kind");
   if (o.arith != AMGB_ARITH_REFERENCE && o.arith != AMGB_ARITH_FAST) throw std::invalid_argument("unknown arithmetic mode");
   if (o.transfer != AMGB_TRANSFER_LINEAR && o.transfer != AMGB_TRANSFER_BILINEAR_2D)
     throw std::invalid_argument("unknown transfer kind");
@@ -2691,6 +2826,14 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
     if (grid_lines(n_rows) < 1)
       throw std::invalid_argument("the bilinear 2-D transfer needs an m x m grid operator, got " + std::to_string(n_rows) +
                                   " rows (not a square number)");
+  }
+  if (o.smoother == AMGB_SMOOTHER_LINE_GS) {
+    if (o.lines != AMGB_LINES_X && o.lines != AMGB_LINES_Y && o.lines != AMGB_LINES_ALTERNATING)
+      throw std::invalid_argument("unknown line direction setting " + std::to_string(o.lines) +
+                                  " (AMGB_LINES_X, AMGB_LINES_Y or AMGB_LINES_ALTERNATING)");
+    if (o.transfer != AMGB_TRANSFER_BILINEAR_2D)
+      throw std::invalid_argument("line Gauss-Seidel needs the bilinear 2-D transfer (AMGB_TRANSFER_BILINEAR_2D): "
+                                  "the coarse levels of the linear transfer are not grids");
   }
   if (!b || !rowidx || !val) throw std::invalid_argument("null argument");
   require_device();
@@ -2730,7 +2873,8 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
   std::vector<FullLevel> full;
   std::vector<Csc> mats;
   const char* force_host = std::getenv("AMGB_HOST_SETUP");
-  if (o.smoother == AMGB_SMOOTHER_JACOBI && !(force_host && std::string(force_host) == "1"))
+  if ((o.smoother == AMGB_SMOOTHER_JACOBI || o.smoother == AMGB_SMOOTHER_LINE_GS) &&
+      !(force_host && std::string(force_host) == "1"))
     h->device_setup = device_build_levels(h.get(), n_rows, colptr, rowidx, val, full);
   if (!h->device_setup) {
     full.clear();
@@ -2906,6 +3050,8 @@ int amgb_hierarchy_create_sharded(amgb_comm* comm, int64_t min_rows_per_rank, in
     if (!comm) throw std::invalid_argument("null communicator");
     if (opt_in && opt_in->transfer == AMGB_TRANSFER_BILINEAR_2D)
       throw std::invalid_argument("the bilinear 2-D transfer is a single-GPU path (no sharded hierarchy)");
+    if (opt_in && opt_in->smoother == AMGB_SMOOTHER_LINE_GS)
+      throw std::invalid_argument("line Gauss-Seidel is a single-GPU path (no sharded hierarchy)");
     CUDA_CHECK(cudaSetDevice(comm->device));
     create_hierarchy(comm, std::max<int64_t>(min_rows_per_rank, 1), n_rows, n_cols, colptr, rowidx, val, b,
                      b_rows, opt_in, out);
@@ -3627,8 +3773,10 @@ int amgb_time_kernel(amgb_hierarchy* h, int level, int kind, int warmup, int rep
       *ms_out = (double)ms / reps;
       return;
     }
-    h->check_level(level, kind >= 2);
+    h->check_level(level, kind == 2 || kind == 3);
     if (kind == 2 || kind == 3) h->require_whole(level);
+    if ((kind == 12 || kind == 13) && h->opt.smoother != AMGB_SMOOTHER_LINE_GS)
+      throw ApiError(AMGB_ESTATE, "kinds 12 and 13 time the passes of a line Gauss-Seidel hierarchy");
     if (kind == 4 || kind == 5) {
       // fused down / up leg of this level; they work on the level state, which is restored
       if (!h->leg_ok(level)) throw ApiError(AMGB_ESTATE, "level has no fused legs");
@@ -3669,11 +3817,14 @@ int amgb_time_kernel(amgb_hierarchy* h, int level, int kind, int warmup, int rep
     Operator& A = *h->ops[level];
     LevelState& S = h->lv[level];
     if (!S.tmp.p) S.tmp.alloc(S.n_vec() + 4);
+    if (kind == 12 || kind == 13)  // the other direction's factors are built on first use
+      A.ensure_line_gs((int)h->m[level], kind == 12 ? lgs::kX : lgs::kY, h->fast_arith(),
+                       "level " + std::to_string(level), s);
     DevBuf<double> scratch_u, scratch_c, scratch_c2;
     scratch_u.alloc(S.n_vec());
     CUDA_CHECK(cudaMemcpyAsync(scratch_u.p, S.u.p, sizeof(double) * S.n_vec(), cudaMemcpyDeviceToDevice, s));
     double* su = scratch_u.p + S.halo_lo;  // first owned row (no halo exchange is timed here)
-    if (kind >= 2) {
+    if (kind == 2 || kind == 3) {
       scratch_c.alloc(h->n[level + 1]);
       scratch_c.zero(s);
       scratch_c2.alloc(h->n[level + 1]);
@@ -3685,6 +3836,8 @@ int amgb_time_kernel(amgb_hierarchy* h, int level, int kind, int warmup, int rep
             A.jacobi(su, S.f.p, h->opt.omega, S.tmp_own(), s);
           else if (h->opt.smoother == AMGB_SMOOTHER_COLOR_GS)
             for (int c = 0; c < A.n_colors; ++c) A.color_pass(c, S.f.p, scratch_u.p, s);
+          else if (h->opt.smoother == AMGB_SMOOTHER_LINE_GS)
+            A.line_gs_half(true, h->opt.lines, h->fast_arith(), S.f.p, scratch_u.p, S.tmp.p, s);
           else
             A.gs_direction(true, S.f.p, scratch_u.p, S.tmp.p, h->opt.gs_mode, s);
           break;
@@ -3703,6 +3856,10 @@ int amgb_time_kernel(amgb_hierarchy* h, int level, int kind, int warmup, int rep
           else
             LAUNCH(dev::k_prolong_add2, blocks_for((h->n[level] + 1) / 2, 256), 256, 0, s, scratch_c.p, 0,
                    (int)h->n[level + 1], scratch_u.p, 0, (int)h->n[level]);
+          break;
+        case 12:
+        case 13:
+          A.line_pass(kind == 12 ? lgs::kX : lgs::kY, 0, h->fast_arith(), S.f.p, scratch_u.p, S.tmp.p, s);
           break;
         default:
           throw std::invalid_argument("unknown kernel kind");

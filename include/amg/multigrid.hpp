@@ -59,7 +59,7 @@ class Multigrid {
     // the two reference checks (multigrid.hpp:165-178) come first, inside the C ABI
     if (compute_error_every_n_iters <= n_iters && (size_t)A.rows() == (size_t)b.rows()) {
       if (!smoother || smoother->device_kind() < 0)
-        throw std::invalid_argument("the GPU driver needs a SparseGaussSeidel, DampedJacobi or "
+        throw std::invalid_argument("the GPU driver needs a SparseGaussSeidel, DampedJacobi, LineGaussSeidel or "
                                     "MulticolorGaussSeidel smoother");
       if (!interpolator || interpolator->device_transfer() < 0)
         throw std::invalid_argument("the GPU driver applies the operators of LinearInterpolator or "
@@ -70,6 +70,7 @@ class Multigrid {
       opt.smoother = smoother->device_kind();
       opt.smoother_iters = (int64_t)smoother->n_iters;
       opt.omega = smoother->device_omega();
+      opt.lines = smoother->device_lines();
     }
     if (!A.isCompressed()) throw std::invalid_argument("A must be compressed (makeCompressed())");
     detail::check(amgb_hierarchy_create((int)A.rows(), (int)A.cols(), A.outerIndexPtr(), A.innerIndexPtr(),

@@ -35,6 +35,8 @@ class SmootherBase {
   // (AMGB_SMOOTHER_*), or -1 for a host-only user smoother the driver cannot use.
   virtual int device_kind() const { return -1; }
   virtual double device_omega() const { return 2.0 / 3.0; }
+  // AMGB_LINES_* of a line smoother (AMGB_SMOOTHER_LINE_GS)
+  virtual int device_lines() const { return AMGB_LINES_X; }
 };
 
 template <class EleType>
@@ -96,6 +98,26 @@ class MulticolorGaussSeidel : public SmootherBase<EleType> {
                                        (int64_t)this->n_iters));
   }
   int device_kind() const override { return AMGB_SMOOTHER_COLOR_GS; }
+};
+
+// zebra line Gauss-Seidel on an m x m grid operator (amgb.h, AMGB_SMOOTHER_LINE_GS): n_iters x (forward
+// half then backward half) per smooth() call; the GPU Multigrid driver needs BilinearInterpolator2D
+template <class EleType>
+class LineGaussSeidel : public SmootherBase<EleType> {
+  int lines_{AMGB_LINES_X};
+
+ public:
+  LineGaussSeidel(size_t n_iters_ = 1, int lines = AMGB_LINES_X) : SmootherBase<EleType>(n_iters_), lines_(lines) {
+    if (lines != AMGB_LINES_X && lines != AMGB_LINES_Y && lines != AMGB_LINES_ALTERNATING)
+      throw std::invalid_argument("`lines` must be AMGB_LINES_X, AMGB_LINES_Y or AMGB_LINES_ALTERNATING but got " +
+                                  std::to_string(lines));
+  }
+  void smooth(const SparseMatrixT<EleType>& A, VectorT<EleType>& u, const VectorT<EleType>& b) override {
+    detail::check(amgb_smooth_line_gs(detail::MirrorCache::instance().get(A), u.data(), b.data(),
+                                      (int64_t)this->n_iters, lines_));
+  }
+  int device_kind() const override { return AMGB_SMOOTHER_LINE_GS; }
+  int device_lines() const override { return lines_; }
 };
 
 namespace detail {
