@@ -103,6 +103,9 @@ SIGNATURES = {
     "amgb_partition_plan": (_i, [_i, np.ctypeslib.ndpointer(dtype=np.int64, flags="C_CONTIGUOUS"), _pi, _i, _l,
                                  C.POINTER(_i), np.ctypeslib.ndpointer(dtype=np.int64, flags="C_CONTIGUOUS"),
                                  _pi, _pi, _pi]),
+    "amgb_partition_plan_2d": (_i, [_i, np.ctypeslib.ndpointer(dtype=np.int64, flags="C_CONTIGUOUS"), _i, _l,
+                                    C.POINTER(_i), np.ctypeslib.ndpointer(dtype=np.int64, flags="C_CONTIGUOUS"),
+                                    _pi, _pi, _pi]),
     "amgb_hierarchy_set_stream": (_i, [_p, _p]),
     "amgb_hierarchy_n_levels": (_i, [_p]),
     "amgb_hierarchy_n_dofs": (_l, [_p, _i]),
@@ -523,6 +526,19 @@ def partition_plan(level_sizes, half_bandwidth, world, min_rows_per_rank):
     starts = np.zeros(L * (world + 1), np.int64)
     lo, hi, gh = np.zeros(L, np.int32), np.zeros(L, np.int32), np.zeros(L, np.int32)
     _check(lib().amgb_partition_plan(L, sizes, bw, world, min_rows_per_rank, C.byref(ns), starts, lo, hi, gh))
+    k = ns.value
+    return k, starts.reshape(L, world + 1)[:k], lo[:k], hi[:k], gh[:k]
+
+
+def partition_plan_2d(lines, world, min_rows_per_rank):
+    """Host-only: (n_sharded, starts[l][g], halo_lo, halo_hi, ghost), all in rows, of the plan of a
+    bilinear 2-D hierarchy with `lines[l]` grid lines on level l (blocks of whole lines)."""
+    L = len(lines)
+    m = np.ascontiguousarray(lines, np.int64)
+    ns = _i()
+    starts = np.zeros(L * (world + 1), np.int64)
+    lo, hi, gh = np.zeros(L, np.int32), np.zeros(L, np.int32), np.zeros(L, np.int32)
+    _check(lib().amgb_partition_plan_2d(L, m, world, min_rows_per_rank, C.byref(ns), starts, lo, hi, gh))
     k = ns.value
     return k, starts.reshape(L, world + 1)[:k], lo[:k], hi[:k], gh[:k]
 

@@ -831,15 +831,17 @@ struct Operator {
                n_coarse);
     });
   }
-  // bilinear transfer of a 2-D hierarchy: this operator is the m_h x m_h grid level, the coarse one m_H x m_H
-  void residual_restrict2d(const double* u, const double* f, int m_h, double* f_coarse, double* u_coarse, int m_H,
-                           cudaStream_t s) const {
-    if (m_H < 1) return;
+  // bilinear transfer of a 2-D hierarchy: this operator is the m_h x m_h grid level (or a block of it whose
+  // first row is global line y_first), the coarse one m_H x m_H; produces coarse lines [Y_begin, Y_end) into
+  // f_coarse / u_coarse, whose line 0 is global line Y_first
+  void residual_restrict2d(const double* u, const double* f, int m_h, int y_first, double* f_coarse,
+                           double* u_coarse, int m_H, int Y_first, int Y_begin, int Y_end, cudaStream_t s) const {
+    if (m_H < 1 || Y_end <= Y_begin) return;
     with_view(rows_of_A(), [&](auto V) {
       auto kern = dev::k_residual_restrict2d<decltype(V)>;
       V.n_rows = n_mat;
-      LAUNCH(kern, dim3(blocks_for(m_H, dev::kRR2X), blocks_for(m_H, dev::kRR2Y)), 256, 0, s, V, u, f, m_h, f_coarse,
-             u_coarse, m_H);
+      LAUNCH(kern, dim3(blocks_for(m_H, dev::kRR2X), blocks_for(Y_end - Y_begin, dev::kRR2Y)), 256, 0, s, V, u, f,
+             m_h, y_first, f_coarse, u_coarse, m_H, Y_first, Y_begin, Y_end);
     });
   }
   int rss_blocks() const { return std::max(1, blocks_for(n, 256)); }
@@ -1393,8 +1395,26 @@ struct amgb_hierarchy {
   void residual_restrict(int l, cudaStream_t s) {
     LevelState& F = lv[l];
     LevelState& C = lv[l + 1];
-    if (bilinear()) {  // (never sharded)
-      ops[l]->residual_restrict2d(F.u.p, F.f.p, (int)m[l], C.f.p, C.u.p, (int)m[l + 1], s);
+    if (bilinear()) {
+      const int m_h = (int)m[l], m_H = (int)m[l + 1];
+      if (!F.sharded) {
+        ops[l]->residual_restrict2d(F.u.p, F.f.p, m_h, 0, C.f.p, C.u.p, m_H, 0, 0, m_H, s);
+        return;
+      }
+      // the block's own coarse lines (and the coarse ghost lines above them when the coarse level is
+      // sharded too) restrict from the own and ghost fine lines, whose residual this rank forms itself
+      exchange(l, F.u.p, s);
+      CUDA_CHECK(cudaMemsetAsync(C.u.p, 0, sizeof(double) * C.u.n, s));
+      const int y0 = (int)(F.s / m_h);
+      if (C.sharded) {
+        const int Y0 = (int)(C.s / m_H);
+        ops[l]->residual_restrict2d(F.u_own(), F.f.p, m_h, y0, C.f.p, C.u_own(), m_H, Y0, Y0, Y0 + C.n_mat / m_H, s);
+      } else {
+        const std::vector<int64_t>& cs = coarse_block_start;
+        ops[l]->residual_restrict2d(F.u_own(), F.f.p, m_h, y0, C.f.p, C.u.p, m_H, 0, (int)(cs[rank()] / m_H),
+                                    (int)(cs[rank() + 1] / m_H), s);
+        gather_coarse_rhs(s);
+      }
       return;
     }
     if (!F.sharded) {
@@ -1419,7 +1439,18 @@ struct amgb_hierarchy {
     LevelState& F = lv[l];
     LevelState& C = lv[l + 1];
     if (bilinear()) {
-      prolong_add2d(C.u.p, F.u.p, l, s);
+      if (!F.sharded) {
+        prolong_add2d(C.u.p, F.u.p, l, s);
+        return;
+      }
+      // the first fine line of the block reads the coarse line below the coarse block (coarse halo)
+      if (C.sharded) exchange(l + 1, C.u.p, s);
+      const int m_h = (int)m[l], m_H = (int)m[l + 1];
+      const int y0 = (int)(F.s / m_h), y1 = (int)(F.e / m_h);
+      const double* e = C.sharded ? C.u_own() : C.u.p;
+      const int Y_first = C.sharded ? (int)(C.s / m_H) : 0;
+      LAUNCH(dev::k_prolong_add2d, dim3(blocks_for(m_h, 256), (unsigned)blocks_for(y1 - y0, 2)), 256, 0, s, e, m_H,
+             Y_first, F.u_own(), m_h, y0, y0, y1);
       return;
     }
     if (C.sharded) exchange(l + 1, C.u.p, s);  // needs e[s_c - 1]
@@ -1434,8 +1465,8 @@ struct amgb_hierarchy {
   // u_l += P_l e on a 2-D hierarchy (e: m_{l+1}^2 coarse values, u: m_l^2 fine values)
   void prolong_add2d(const double* e, double* u, int l, cudaStream_t s) const {
     if (m[l] < 1) return;
-    LAUNCH(dev::k_prolong_add2d, dim3(blocks_for(m[l], 256), (unsigned)blocks_for(m[l], 2)), 256, 0, s, e, (int)m[l + 1], u,
-           (int)m[l]);
+    LAUNCH(dev::k_prolong_add2d, dim3(blocks_for(m[l], 256), (unsigned)blocks_for(m[l], 2)), 256, 0, s, e, (int)m[l + 1], 0,
+           u, (int)m[l], 0, 0, (int)m[l]);
   }
   // f_c = R_l r on a 2-D hierarchy
   void restrict2d(const double* r, double* f_c, int l, cudaStream_t s) const {
@@ -2931,7 +2962,7 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
     // sharding (they run as streaming legs on the rank's window); the levels below, a few
     // hundred thousand rows at most, are agglomerated.
     int max_sharded = 1 << 30;
-    if ((o.fuse & 4) && o.smoother == AMGB_SMOOTHER_JACOBI && (o.smoother_iters == 1 || o.smoother_iters == 2)) {
+    if ((h->opt.fuse & 4) && o.smoother == AMGB_SMOOTHER_JACOBI && (o.smoother_iters == 1 || o.smoother_iters == 2)) {
       max_sharded = 0;
       for (int l = 0; l + 1 < L; ++l) {
         const std::vector<int>& offs = level_off[l];
@@ -2945,12 +2976,18 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
       }
       if (max_sharded == 0) max_sharded = 1 << 30;  // no streamable level: the per-operator kernels shard as before
     }
-    h->plan = make_partition_plan(h->n, half_bw, world, min_rows_per_rank, max_sharded);
+    h->plan = h->bilinear() ? make_partition_plan_2d(h->m, world, min_rows_per_rank)
+                            : make_partition_plan(h->n, half_bw, world, min_rows_per_rank, max_sharded);
     h->n_sharded = h->plan.n_sharded;
     if (h->n_sharded > 0) {
+      // the first replicated level's rows each rank restricts into: half the fine rows (1-D), or the
+      // coarse lines from half the fine block's first line (2-D)
+      const int ns = h->n_sharded;
       h->coarse_block_start.resize(world + 1);
       for (int g = 0; g <= world; ++g)
-        h->coarse_block_start[g] = (g == world) ? h->n[h->n_sharded] : h->plan.start[h->n_sharded - 1][g] / 2;
+        h->coarse_block_start[g] = (g == world)      ? h->n[ns]
+                                   : h->bilinear() ? h->plan.start[ns - 1][g] / h->m[ns - 1] / 2 * h->m[ns]
+                                                   : h->plan.start[ns - 1][g] / 2;
     }
   }
 
@@ -2963,7 +3000,7 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
     S.n_global = h->n[l];
     h->ops[l].reset(new Operator());
     const bool want_window =
-        (o.fuse & 4) && o.smoother == AMGB_SMOOTHER_JACOBI && (o.smoother_iters == 1 || o.smoother_iters == 2);
+        (h->opt.fuse & 4) && o.smoother == AMGB_SMOOTHER_JACOBI && (o.smoother_iters == 1 || o.smoother_iters == 2);
     if (l < h->n_sharded) {
       S.sharded = true;
       S.s = h->plan.start[l][g];
@@ -3048,10 +3085,12 @@ int amgb_hierarchy_create_sharded(amgb_comm* comm, int64_t min_rows_per_rank, in
                                   int64_t b_rows, const amgb_options* opt_in, amgb_hierarchy** out) {
   return guarded([&] {
     if (!comm) throw std::invalid_argument("null communicator");
-    if (opt_in && opt_in->transfer == AMGB_TRANSFER_BILINEAR_2D)
-      throw std::invalid_argument("the bilinear 2-D transfer is a single-GPU path (no sharded hierarchy)");
     if (opt_in && opt_in->smoother == AMGB_SMOOTHER_LINE_GS)
-      throw std::invalid_argument("line Gauss-Seidel is a single-GPU path (no sharded hierarchy)");
+      throw std::invalid_argument("line Gauss-Seidel is a single-GPU path (no sharded hierarchy): every pass walks "
+                                  "whole grid lines, so row blocks would not shorten it");
+    if (opt_in && opt_in->transfer == AMGB_TRANSFER_BILINEAR_2D && comm->world < 2)
+      throw std::invalid_argument("a sharded bilinear 2-D hierarchy needs a communicator of at least two ranks "
+                                  "(nothing to shard: use amgb_hierarchy_create)");
     CUDA_CHECK(cudaSetDevice(comm->device));
     create_hierarchy(comm, std::max<int64_t>(min_rows_per_rank, 1), n_rows, n_cols, colptr, rowidx, val, b,
                      b_rows, opt_in, out);
@@ -3120,6 +3159,28 @@ int amgb_partition_plan(int n_levels, const int64_t* level_sizes, const int* hal
     std::vector<int64_t> sizes(level_sizes, level_sizes + n_levels);
     std::vector<int> bw(half_bandwidth, half_bandwidth + n_levels);
     PartitionPlan P = make_partition_plan(sizes, bw, world, std::max<int64_t>(min_rows_per_rank, 1));
+    *n_sharded = P.n_sharded;
+    for (int l = 0; l < P.n_sharded; ++l) {
+      if (starts)
+        for (int g = 0; g <= world; ++g) starts[(size_t)l * (world + 1) + g] = P.start[l][g];
+      if (halo_lo) halo_lo[l] = P.halo_lo[l];
+      if (halo_hi) halo_hi[l] = P.halo_hi[l];
+      if (ghost) ghost[l] = P.ghost[l];
+    }
+  });
+}
+int amgb_partition_plan_2d(int n_levels, const int64_t* lines, int world, int64_t min_rows_per_rank, int* n_sharded,
+                           int64_t* starts, int* halo_lo, int* halo_hi, int* ghost) {
+  return guarded([&] {
+    if (!lines || !n_sharded || n_levels < 1 || world < 1) throw std::invalid_argument("bad plan arguments");
+    std::vector<int64_t> m(lines, lines + n_levels);
+    if (m[0] < 1 || m[0] * m[0] > std::numeric_limits<int>::max())
+      throw std::invalid_argument("bad plan arguments: level 0 must have 1 .. 46340 lines");
+    for (int l = 1; l < n_levels; ++l)
+      if (m[l] < 1 || m[l] != coarse_lines_2d(m[l - 1]))
+        throw std::invalid_argument("bad plan arguments: level " + std::to_string(l) + " has " + std::to_string(m[l]) +
+                                    " lines, the bilinear transfer gives " + std::to_string(coarse_lines_2d(m[l - 1])));
+    PartitionPlan P = make_partition_plan_2d(m, world, std::max<int64_t>(min_rows_per_rank, 1));
     *n_sharded = P.n_sharded;
     for (int l = 0; l < P.n_sharded; ++l) {
       if (starts)
@@ -3846,7 +3907,8 @@ int amgb_time_kernel(amgb_hierarchy* h, int level, int kind, int warmup, int rep
           break;
         case 2:
           if (h->bilinear())
-            A.residual_restrict2d(scratch_u.p, S.f.p, (int)h->m[level], scratch_c2.p, scratch_c.p, (int)h->m[level + 1], s);
+            A.residual_restrict2d(scratch_u.p, S.f.p, (int)h->m[level], 0, scratch_c2.p, scratch_c.p, (int)h->m[level + 1],
+                                  0, 0, (int)h->m[level + 1], s);
           else
             A.residual_restrict(scratch_u.p, S.f.p, scratch_c2.p, scratch_c.p, (int)h->n[level + 1], s);
           break;

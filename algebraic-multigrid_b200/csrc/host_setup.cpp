@@ -475,6 +475,47 @@ PartitionPlan make_partition_plan(const std::vector<int64_t>& level_sizes,
   return P;
 }
 
+PartitionPlan make_partition_plan_2d(const std::vector<int64_t>& lines, int world, int64_t min_rows_per_rank) {
+  PartitionPlan P;
+  P.world = world;
+  P.n_levels = static_cast<int>(lines.size());
+  for (int64_t m : lines) P.n.push_back(m * m);
+  if (world <= 1) return P;
+  int ns = 0;
+  while (ns + 1 < P.n_levels && P.n[ns] / world >= min_rows_per_rank) ++ns;
+  for (; ns > 0; --ns) {
+    const int64_t align = 1ll << ns;
+    P.start.assign(ns, std::vector<int64_t>(world + 1, 0));
+    P.halo_lo.assign(ns, 0);
+    P.halo_hi.assign(ns, 0);
+    P.ghost.assign(ns, 0);
+    bool ok = true;
+    int64_t ghost_lines = 0;
+    for (int l = ns - 1; l >= 0; --l) {
+      ghost_lines = 2 * ghost_lines + 1;
+      const int64_t m = lines[l];
+      P.ghost[l] = static_cast<int>(ghost_lines * m);
+      P.halo_lo[l] = static_cast<int>(m + 2);
+      P.halo_hi[l] = static_cast<int>((ghost_lines + 1) * m + 2);
+      for (int g = 0; g <= world; ++g) {
+        const int64_t y0 = (lines[0] * g / world) / align * align;
+        P.start[l][g] = (g == world) ? P.n[l] : (y0 >> l) * m;
+      }
+      for (int g = 0; g < world; ++g)
+        ok = ok && P.start[l][g + 1] - P.start[l][g] >= std::max(P.halo_lo[l], P.halo_hi[l]);
+    }
+    if (ok) break;
+  }
+  P.n_sharded = ns;
+  if (ns == 0) {
+    P.start.clear();
+    P.halo_lo.clear();
+    P.halo_hi.clear();
+    P.ghost.clear();
+  }
+  return P;
+}
+
 // ------------------------------------------------------------------ GS schedule
 
 Schedule gs_schedule(const Csc& M, bool forward) {

@@ -127,6 +127,16 @@ struct PartitionPlan {
 PartitionPlan make_partition_plan(const std::vector<int64_t>& level_sizes,
                                   const std::vector<int>& half_bandwidth, int world,
                                   int64_t min_rows_per_rank, int max_sharded = 1 << 30);
+// Plan of a bilinear 2-D hierarchy (m_l x m_l grids, m_{l+1} = m_l / 2): blocks of whole grid lines.
+// Level 0 gets the line starts Y0(g) = floor(m_0 g / world) rounded down to a multiple of 2^n_sharded,
+// level l the lines Y0(g) >> l (the last rank ends at m_l); start = line * m_l, so a coarse block
+// starts exactly at half its fine block's first line.  Coarse line J restricts fine lines 2J..2J+2,
+// hence ghost lines ghost_{ns-1} = 1, ghost_l = 2 ghost_{l+1} + 1; in rows ghost = lines * m_l,
+// halo_lo = m_l + 2 (the +-(m_l + 1) stencil plus a margin) and halo_hi = (ghost lines + 1) m_l + 2.
+// Level l is sharded while m_l^2 / world >= min_rows_per_rank (never the coarsest level), and
+// n_sharded shrinks until every block holds at least max(halo_lo, halo_hi) rows.
+PartitionPlan make_partition_plan_2d(const std::vector<int64_t>& lines_per_level, int world,
+                                     int64_t min_rows_per_rank);
 
 // ---- Gauss-Seidel wavefront schedule on the pruned dependency DAG ----
 // forward: row k depends on rows j<k with M(j,k) != 0 (column k of M used as

@@ -630,22 +630,30 @@ __global__ void __launch_bounds__(256) k_restrict2d(const double* __restrict__ r
 // fine points under the tile in shared memory (k_residual's per-row arithmetic) and restricts from
 // there, so r never reaches HBM.  Neighbouring tiles share one fine line / column: 17 x 129 residuals
 // for 16 x 128 distinct ones, 7 % formed twice.
+// Window: the block produces the coarse lines [Y_begin, Y_end) (global line numbers); local line 0 of
+// u, f and the operator rows is global fine line y_first, local line 0 of f_coarse / u_coarse global
+// coarse line Y_first.  Residuals are formed on the fine lines [2 Y_begin, 2 Y_end] only (those the
+// coarse lines restrict from), so a rank of a sharded level reads its own lines, the ghost lines above
+// them and one line of u either side.  The whole level is y_first = Y_first = Y_begin = 0, Y_end = m_H
+// (2 m_H + 1 >= m_h: every line, as before).
 constexpr int kRR2X = 64, kRR2Y = 8;
 template <class M>
 __global__ void __launch_bounds__(256) k_residual_restrict2d(M A, const double* __restrict__ u,
-                                                             const double* __restrict__ f, int m_h,
+                                                             const double* __restrict__ f, int m_h, int y_first,
                                                              double* __restrict__ f_coarse,
-                                                             double* __restrict__ u_coarse, int m_H) {
+                                                             double* __restrict__ u_coarse, int m_H, int Y_first,
+                                                             int Y_begin, int Y_end) {
   constexpr int FX = 2 * kRR2X + 1, FY = 2 * kRR2Y + 1;
   __shared__ double r[FY * FX];
-  const int X0 = blockIdx.x * kRR2X, Y0 = blockIdx.y * kRR2Y;
+  const int X0 = blockIdx.x * kRR2X, Y0 = Y_begin + blockIdx.y * kRR2Y;
   const int x0 = 2 * X0, y0 = 2 * Y0;
+  const int y_end = min(m_h, 2 * Y_end + 1);
   for (int p = threadIdx.x; p < FY * FX; p += blockDim.x) {
     const int fy = p / FX, fx = p - fy * FX;
     const int y = y0 + fy, x = x0 + fx;
     double v = 0.0;
-    if (y < m_h && x < m_h) {
-      const int row = y * m_h + x;
+    if (y < y_end && x < m_h) {
+      const int row = (y - y_first) * m_h + x;
       v = row_residual(A, row, row, u, f[row]);
     }
     r[p] = v;
@@ -654,7 +662,7 @@ __global__ void __launch_bounds__(256) k_residual_restrict2d(M A, const double* 
   for (int p = threadIdx.x; p < kRR2Y * kRR2X; p += blockDim.x) {
     const int ty = p / kRR2X, tx = p - ty * kRR2X;
     const int Y = Y0 + ty, X = X0 + tx;
-    if (Y >= m_H || X >= m_H) continue;
+    if (Y >= Y_end || X >= m_H) continue;
     double acc = 0.0;
 #pragma unroll
     for (int a = 0; a < 3; ++a) {
@@ -665,7 +673,7 @@ __global__ void __launch_bounds__(256) k_residual_restrict2d(M A, const double* 
         acc = __dadd_rn(acc, __dmul_rn(bl_w(a) * bl_w(b), r[(2 * ty + a) * FX + 2 * tx + b]));
       }
     }
-    const size_t J = (size_t)Y * m_H + X;
+    const size_t J = (size_t)(Y - Y_first) * m_H + X;
     f_coarse[J] = acc;
     if (u_coarse) u_coarse[J] = 0.0;
   }
@@ -674,7 +682,8 @@ __global__ void __launch_bounds__(256) k_residual_restrict2d(M A, const double* 
 // (P e) at fine point (y, x): fine coordinate y takes coarse Y = (y - 1) / 2 with weight 1 when odd, and
 // Y = y / 2 - 1, y / 2 (those inside the coarse grid) with weight .5 each when even; the terms are summed
 // in ascending coarse index (Y-major).  Fully unrolled and predicated, so all loads are independent.
-__device__ __forceinline__ double prolong2d_at(const double* __restrict__ e, int m_H, int y, int x) {
+// e points at global coarse line Y_first (lines below it may be read from a halo: signed offsets).
+__device__ __forceinline__ double prolong2d_at(const double* __restrict__ e, int m_H, int Y_first, int y, int x) {
   const int ylo = (y & 1) ? (y >> 1) : max((y >> 1) - 1, 0), yhi = (y & 1) ? (y >> 1) : min(y >> 1, m_H - 1);
   const int xlo = (x & 1) ? (x >> 1) : max((x >> 1) - 1, 0), xhi = (x & 1) ? (x >> 1) : min(x >> 1, m_H - 1);
   const double w = ((y & 1) ? 1.0 : 0.5) * ((x & 1) ? 1.0 : 0.5);
@@ -683,7 +692,7 @@ __device__ __forceinline__ double prolong2d_at(const double* __restrict__ e, int
   for (int i = 0; i < 2; ++i)
 #pragma unroll
     for (int j = 0; j < 2; ++j)
-      v[2 * i + j] = (ylo + i <= yhi && xlo + j <= xhi) ? e[(size_t)(ylo + i) * m_H + xlo + j] : 0.0;
+      v[2 * i + j] = (ylo + i <= yhi && xlo + j <= xhi) ? e[(long long)(ylo + i - Y_first) * m_H + xlo + j] : 0.0;
   double acc = 0.0;
 #pragma unroll
   for (int i = 0; i < 2; ++i)
@@ -693,16 +702,19 @@ __device__ __forceinline__ double prolong2d_at(const double* __restrict__ e, int
   return acc;
 }
 
-// u += P e: a thread owns fine column x of the two fine lines 2 blockIdx.y, 2 blockIdx.y + 1 (an even and
-// an odd line, which share their coarse lines), with every load issued before the first add.
-__global__ void __launch_bounds__(256) k_prolong_add2d(const double* __restrict__ e, int m_H,
-                                                       double* __restrict__ u, int m_h) {
-  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = 2 * blockIdx.y;
+// u += P e on the fine lines [y_begin, y_end) (y_begin even): a thread owns fine column x of the two
+// fine lines y_begin + 2 blockIdx.y and the one after it (an even and an odd line, which share their
+// coarse lines), with every load issued before the first add.  Local line 0 of u is global fine line
+// y_first, of e global coarse line Y_first; the whole level is y_first = Y_first = y_begin = 0, y_end = m_h.
+__global__ void __launch_bounds__(256) k_prolong_add2d(const double* __restrict__ e, int m_H, int Y_first,
+                                                       double* __restrict__ u, int m_h, int y_first, int y_begin,
+                                                       int y_end) {
+  const int x = blockIdx.x * blockDim.x + threadIdx.x, y = y_begin + 2 * blockIdx.y;
   if (x >= m_h) return;
-  const bool two = y + 1 < m_h;
-  const size_t k = (size_t)y * m_h + x;
+  const bool two = y + 1 < y_end;
+  const size_t k = (size_t)(y - y_first) * m_h + x;
   const double u0 = u[k], u1 = two ? u[k + m_h] : 0.0;
-  const double a0 = prolong2d_at(e, m_H, y, x), a1 = two ? prolong2d_at(e, m_H, y + 1, x) : 0.0;
+  const double a0 = prolong2d_at(e, m_H, Y_first, y, x), a1 = two ? prolong2d_at(e, m_H, Y_first, y + 1, x) : 0.0;
   u[k] = __dadd_rn(u0, a0);
   if (two) u[k + m_h] = __dadd_rn(u1, a1);
 }
