@@ -23,7 +23,7 @@ LINES_X, LINES_Y, LINES_ALTERNATING = 0, 1, 2
 GS_AUTO, GS_LEVELSCHED, GS_LINESCAN = 0, 1, 2
 GS_KERNEL_FRONTS, GS_KERNEL_LINESCAN, GS_KERNEL_WAVE = 0, 1, 2
 ARITH_REFERENCE, ARITH_FAST = 0, 1
-TRANSFER_LINEAR, TRANSFER_BILINEAR_2D = 0, 1
+TRANSFER_LINEAR, TRANSFER_BILINEAR_2D, TRANSFER_SMOOTHED_AGGREGATION = 0, 1, 2
 
 _i, _l, _d, _p = C.c_int, C.c_int64, C.c_double, C.c_void_p
 _pd = np.ctypeslib.ndpointer(dtype=np.float64, flags="C_CONTIGUOUS")
@@ -31,12 +31,21 @@ _pi = np.ctypeslib.ndpointer(dtype=np.int32, flags="C_CONTIGUOUS")
 
 
 class Options(C.Structure):
+    """amgb_options up to `lines`."""
     _fields_ = [("n_levels", _i), ("tolerance", _d),
                 ("compute_error_every_n_iters", _l), ("n_iters", _l),
                 ("smoother", _i), ("smoother_iters", _l), ("omega", _d),
                 ("gs_mode", _i), ("use_graph", _i),
                 ("skip_dead_coarse_smooth", _i), ("fuse", _i), ("arith", _i),
                 ("transfer", _i), ("lines", _i)]
+
+
+class FullOptions(C.Structure):
+    """The whole amgb_options: Options, then the fields appended after `lines`.  sizeof(Options) is a
+    multiple of 8, which is where the C struct's next double starts, so the layouts agree; the fields of
+    Options are reachable directly (o.n_levels)."""
+    _anonymous_ = ("base",)
+    _fields_ = [("base", Options), ("strength", _d)]
 
 
 class AmgbError(RuntimeError):
@@ -66,6 +75,7 @@ SIGNATURES = {
     "amgb_bilinear_coarse_lines": (_l, [_l]),
     "amgb_bilinear_nnz": (_l, [_l, _l]),
     "amgb_bilinear_make_operators": (_i, [_l, _l, _pi, _pi, _pd, _pi, _pi, _pd]),
+    "amgb_sa_aggregate": (_i, [_i, _pi, _pi, _pd, _d, _pi, C.POINTER(_l)]),
     "amgb_linear_restrict": (_i, [_l, _l, _pd, _pd]),
     "amgb_linear_prolong": (_i, [_l, _l, _pd, _pd]),
     "amgb_csc_spmv": (_i, [_i, _i, _pi, _pi, _pd, _pd, _pd]),
@@ -84,16 +94,17 @@ SIGNATURES = {
     "amgb_matrix_stream_bytes": (_l, [_p, _i]),
     "amgb_matrix_gs_kernel": (_i, [_p, _i]),
     "amgb_selftest_division": (_i, [_l, C.c_uint64, C.POINTER(_l)]),
-    "amgb_options_default": (None, [C.POINTER(Options)]),
-    "amgb_hierarchy_create": (_i, [_i, _i, _pi, _pi, _pd, _pd, _l, C.POINTER(Options),
+    "amgb_options_default": (None, [C.POINTER(FullOptions)]),
+    "amgb_hierarchy_create": (_i, [_i, _i, _pi, _pi, _pd, _pd, _l, C.POINTER(FullOptions),
                                    C.POINTER(_p)]),
     "amgb_hierarchy_destroy": (_i, [_p]),
     "amgb_hierarchy_transfer": (_i, [_p]),
+    "amgb_hierarchy_get_transfer": (_i, [_p, _i, C.POINTER(_l), _p, _p, _p]),
     "amgb_comm_unique_id_bytes": (_i, []),
     "amgb_comm_get_unique_id": (_i, [_p]),
     "amgb_comm_create": (_i, [_p, _i, _i, C.POINTER(_p)]),
     "amgb_comm_destroy": (_i, [_p]),
-    "amgb_hierarchy_create_sharded": (_i, [_p, _l, _i, _i, _pi, _pi, _pd, _pd, _l, C.POINTER(Options),
+    "amgb_hierarchy_create_sharded": (_i, [_p, _l, _i, _i, _pi, _pi, _pd, _pd, _l, C.POINTER(FullOptions),
                                            C.POINTER(_p)]),
     "amgb_hierarchy_n_sharded_levels": (_i, [_p]),
     "amgb_hierarchy_local_range": (_i, [_p, _i, C.POINTER(_l), C.POINTER(_l)]),
@@ -307,6 +318,41 @@ class BilinearInterpolator2D(LinearInterpolator):
         _check(lib().amgb_bilinear_make_operators(m_h, m_H, Pc, Pr, Pv, Rc, Rr, Rv))
         self._P[level] = CscMatrix(n_h, n_H, Pc, Pr, Pv)
         self._R[level] = CscMatrix(n_H, n_h, Rc, Rr, Rv)
+
+
+class SmoothedAggregation(LinearInterpolator):
+    """Smoothed-aggregation coarsening (TRANSFER_SMOOTHED_AGGREGATION, include/amgb.h): aggregates of
+    strongly coupled rows (threshold `strength`), P = (I - w D^-1 A) T.  Needs no grid, so it runs on
+    rectangular grids, permuted numberings, wide stencils and unstructured matrices.  n_levels is a cap:
+    the hierarchy coarsens while a level has more than 200 rows, and stops at a coarse level whose
+    aggregation does not reduce it.  The aggregation depends on A, so
+    Multigrid fills the P and R slots from the hierarchy it built; make_operators cannot."""
+
+    transfer = TRANSFER_SMOOTHED_AGGREGATION
+
+    def __init__(self, n_levels, strength=0.08):
+        super().__init__(n_levels)
+        self.strength = float(strength)
+
+    def make_operators(self, n_h, n_H, level):
+        raise NotImplementedError("SmoothedAggregation's operators depend on A: Multigrid builds them")
+
+
+def sa_aggregate(A, strength=0.08):
+    """(agg, n_aggregates) of the smoothed-aggregation rule on host matrix A (host only)."""
+    agg = np.empty(A.cols, np.int32)
+    k = _l()
+    _check(lib().amgb_sa_aggregate(A.cols, A.colptr, A.rowidx, A.val, float(strength), agg, C.byref(k)))
+    return agg, k.value
+
+
+def _transpose(M):
+    """CSC of M^T (an index permutation: entries keep their values, rows stay ascending)."""
+    order = np.argsort(M.rowidx, kind="stable")
+    colptr = np.zeros(M.rows + 1, np.int64)
+    np.add.at(colptr, M.rowidx.astype(np.int64) + 1, 1)
+    cols = np.repeat(np.arange(M.cols, dtype=np.int32), np.diff(M.colptr))
+    return CscMatrix(M.cols, M.rows, np.cumsum(colptr), cols[order], M.val[order])
 
 
 class DeviceMatrix:
@@ -551,7 +597,7 @@ class Multigrid:
                  skip_dead_coarse_smooth=True, comm=None, min_rows_per_rank=1 << 18, fuse=None,
                  arith=ARITH_REFERENCE):
         self.interpolator, self.smoother = interpolator, smoother
-        o = Options()
+        o = FullOptions()
         lib().amgb_options_default(C.byref(o))
         o.n_levels = n_levels
         o.tolerance = tolerance
@@ -568,6 +614,7 @@ class Multigrid:
         o.arith = int(arith)
         o.transfer = int(getattr(interpolator, "transfer", TRANSFER_LINEAR))
         o.lines = int(getattr(smoother, "lines", LINES_X))
+        o.strength = float(getattr(interpolator, "strength", o.strength))
         b = _f64(b)
         h = _p()
         if comm is None:
@@ -579,12 +626,17 @@ class Multigrid:
                                                        C.byref(h)))
         self.comm = comm
         self.h = h
-        self.n_levels = n_levels
+        self.n_levels = lib().amgb_hierarchy_n_levels(h)  # (a cap for smoothed aggregation)
         self.display_error = False
         # the driver fills the interpolator's slots like the reference does (multigrid.hpp:218)
         if interpolator is not None:
-            for l in range(1, n_levels):
-                interpolator.make_operators(self.get_n_dofs(l - 1), self.get_n_dofs(l), l - 1)
+            for l in range(1, self.n_levels):
+                if o.transfer == TRANSFER_SMOOTHED_AGGREGATION:
+                    P = self.get_transfer(l - 1)
+                    interpolator.set_level_to_P(l - 1, P)
+                    interpolator.set_level_to_R(l - 1, _transpose(P))
+                else:
+                    interpolator.make_operators(self.get_n_dofs(l - 1), self.get_n_dofs(l), l - 1)
 
     def __del__(self):
         if getattr(self, "h", None) and _lib is not None:
@@ -598,6 +650,16 @@ class Multigrid:
     def transfer(self):
         """TRANSFER_* the hierarchy was built with."""
         return lib().amgb_hierarchy_transfer(self.h)
+
+    def get_transfer(self, level):
+        """P of `level` (n_level x n_level+1) as the hierarchy applies it."""
+        nnz = _l()
+        _check(lib().amgb_hierarchy_get_transfer(self.h, level, C.byref(nnz), None, None, None))
+        nf, nc = self.get_n_dofs(level), self.get_n_dofs(level + 1)
+        colptr, rowidx, val = np.empty(nc + 1, np.int32), np.empty(nnz.value, np.int32), np.empty(nnz.value)
+        _check(lib().amgb_hierarchy_get_transfer(self.h, level, C.byref(nnz), colptr.ctypes.data,
+                                                 rowidx.ctypes.data, val.ctypes.data))
+        return CscMatrix(nf, nc, colptr, rowidx, val)
 
     def get_tolerance(self):
         return lib().amgb_hierarchy_tolerance(self.h)

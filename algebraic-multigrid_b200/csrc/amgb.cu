@@ -25,6 +25,7 @@
 #include "line_gs.cuh"
 #include "mid_levels.cuh"
 #include "setup_dia.cuh"
+#include "transfer_sa.cuh"
 #include "stream_leg_api.hpp"
 #include "nccl_dyn.hpp"
 
@@ -880,6 +881,7 @@ void options_default(amgb_options* o) {
   o->arith = AMGB_ARITH_REFERENCE;
   o->transfer = AMGB_TRANSFER_LINEAR;
   o->lines = AMGB_LINES_X;
+  o->strength = 0.08;
   // the C++ mirror of the reference's headers has no argument for it: AMGB_ARITH=fast selects the fast
   // arithmetic for hierarchies created with the default options
   if (const char* a = std::getenv("AMGB_ARITH"))
@@ -940,6 +942,11 @@ struct amgb_hierarchy {
   std::vector<int64_t> n;
   std::vector<int64_t> m;  // grid lines per level of a 2-D hierarchy (n[l] = m[l]^2), empty otherwise
   bool bilinear() const { return opt.transfer == AMGB_TRANSFER_BILINEAR_2D; }
+  bool sa() const { return opt.transfer == AMGB_TRANSFER_SMOOTHED_AGGREGATION; }
+  // smoothed aggregation: P_l on the host, and on the device the rows of R_l = P_l^T (the CSC columns
+  // of P_l) and the rows of P_l, both SELL-32
+  std::vector<Csc> sa_P;
+  std::vector<DevSell> sa_R_rows, sa_P_rows;
   std::vector<std::unique_ptr<Operator>> ops;
   std::vector<LevelState> lv;
   DevBuf<double> partial, scalar;
@@ -1395,6 +1402,11 @@ struct amgb_hierarchy {
   void residual_restrict(int l, cudaStream_t s) {
     LevelState& F = lv[l];
     LevelState& C = lv[l + 1];
+    if (sa()) {  // residual into the level's scratch vector, then the restriction (transfer_sa.cuh)
+      ops[l]->residual(F.u.p, F.f.p, F.tmp.p, s);
+      restrict_sa(F.tmp.p, C.f.p, C.u.p, l, s);
+      return;
+    }
     if (bilinear()) {
       const int m_h = (int)m[l], m_H = (int)m[l + 1];
       if (!F.sharded) {
@@ -1438,6 +1450,10 @@ struct amgb_hierarchy {
   void prolong_add(int l, cudaStream_t s) {
     LevelState& F = lv[l];
     LevelState& C = lv[l + 1];
+    if (sa()) {
+      prolong_add_sa(C.u.p, F.u.p, l, s);
+      return;
+    }
     if (bilinear()) {
       if (!F.sharded) {
         prolong_add2d(C.u.p, F.u.p, l, s);
@@ -1474,8 +1490,23 @@ struct amgb_hierarchy {
     LAUNCH(dev::k_restrict2d, dim3(blocks_for(m[l + 1], 256), (unsigned)m[l + 1]), 256, 0, s, r, (int)m[l], f_c,
            (int)m[l + 1]);
   }
+  // f_c = R_l r (and u_c = 0 unless u_c is null) on a smoothed-aggregation hierarchy
+  void restrict_sa(const double* r, double* f_c, double* u_c, int l, cudaStream_t s) const {
+    const DevSell& R = sa_R_rows[l];
+    if (R.n_rows < 1) return;
+    if (fast_arith()) LAUNCH(sa::k_restrict_sa<true>, blocks_for(R.n_rows, 256), 256, 0, s, R.view(), r, f_c, u_c);
+    else LAUNCH(sa::k_restrict_sa<false>, blocks_for(R.n_rows, 256), 256, 0, s, R.view(), r, f_c, u_c);
+  }
+  // u_l += P_l e on a smoothed-aggregation hierarchy
+  void prolong_add_sa(const double* e, double* u, int l, cudaStream_t s) const {
+    const DevSell& P = sa_P_rows[l];
+    if (P.n_rows < 1) return;
+    if (fast_arith()) LAUNCH(sa::k_prolong_add_sa<true>, blocks_for(P.n_rows, 256), 256, 0, s, P.view(), e, u);
+    else LAUNCH(sa::k_prolong_add_sa<false>, blocks_for(P.n_rows, 256), 256, 0, s, P.view(), e, u);
+  }
   // P_l of this hierarchy's transfer kind (host setup)
   Csc prolongation(int l) const {
+    if (sa()) return sa_P[l];
     return bilinear() ? make_prolongation_2d(m[l], m[l + 1]) : make_prolongation(n[l], n[l + 1]);
   }
   void coarse_solve(cudaStream_t s) {  // multigrid.hpp:287-288
@@ -2333,6 +2364,15 @@ int amgb_bilinear_make_operators(int64_t m_h, int64_t m_H, int* P_colptr, int* P
     std::memcpy(R_val, R.val.data(), R.val.size() * sizeof(double));
   });
 }
+int amgb_sa_aggregate(int n, const int* colptr, const int* rowidx, const double* val, double theta, int* agg,
+                      int64_t* n_aggregates) {
+  return guarded([&] {
+    if (n < 0 || !colptr || !rowidx || !val || !agg || !n_aggregates) throw std::invalid_argument("null argument");
+    std::vector<int> a;
+    *n_aggregates = sa_aggregate(csc_from_arrays(n, n, colptr, rowidx, val), theta, a);
+    std::memcpy(agg, a.data(), a.size() * sizeof(int));
+  });
+}
 int amgb_linear_restrict(int64_t n_h, int64_t n_H, const double* r, double* out) {
   return guarded([&] {
     if (!r || !out || n_h < 0 || n_H < 0) throw std::invalid_argument("bad transfer arguments");
@@ -2851,8 +2891,16 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
   if (n_rows != n_cols) throw std::invalid_argument("A must be square");
   if (o.smoother < 0 || o.smoother > 3) throw std::invalid_argument("unknown smoother kind");
   if (o.arith != AMGB_ARITH_REFERENCE && o.arith != AMGB_ARITH_FAST) throw std::invalid_argument("unknown arithmetic mode");
-  if (o.transfer != AMGB_TRANSFER_LINEAR && o.transfer != AMGB_TRANSFER_BILINEAR_2D)
+  if (o.transfer != AMGB_TRANSFER_LINEAR && o.transfer != AMGB_TRANSFER_BILINEAR_2D &&
+      o.transfer != AMGB_TRANSFER_SMOOTHED_AGGREGATION)
     throw std::invalid_argument("unknown transfer kind");
+  if (o.transfer == AMGB_TRANSFER_SMOOTHED_AGGREGATION) {
+    if (!(o.strength >= 0.0))
+      throw std::invalid_argument("smoothed aggregation: strength must be >= 0, got " + std::to_string(o.strength));
+    if (comm)
+      throw std::invalid_argument("smoothed aggregation has no sharded hierarchy: aggregate numbering does not give "
+                                  "row blocks whose halos come from ranks +-1 only (use amgb_hierarchy_create)");
+  }
   if (o.transfer == AMGB_TRANSFER_BILINEAR_2D) {
     if (grid_lines(n_rows) < 1)
       throw std::invalid_argument("the bilinear 2-D transfer needs an m x m grid operator, got " + std::to_string(n_rows) +
@@ -2864,7 +2912,7 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
                                   " (AMGB_LINES_X, AMGB_LINES_Y or AMGB_LINES_ALTERNATING)");
     if (o.transfer != AMGB_TRANSFER_BILINEAR_2D)
       throw std::invalid_argument("line Gauss-Seidel needs the bilinear 2-D transfer (AMGB_TRANSFER_BILINEAR_2D): "
-                                  "the coarse levels of the linear transfer are not grids");
+                                  "the coarse levels of the linear and smoothed-aggregation transfers are not grids");
   }
   if (!b || !rowidx || !val) throw std::invalid_argument("null argument");
   require_device();
@@ -2873,13 +2921,20 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
   h->opt = o;
   // fuse bits 1-7 (folded prolongation, fused legs, coarse tail, mid levels, compressed formats) hard-code
   // the 1-D transfer; a 2-D hierarchy runs the per-operator cycle with the zero-guess first sweep only
-  if (h->bilinear()) h->opt.fuse &= 1;
+  if (h->bilinear() || h->sa()) h->opt.fuse &= 1;
   h->L = o.n_levels;
   h->comm = comm;
   CUDA_CHECK(cudaGetDevice(&h->device));
   CUDA_CHECK(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
   h->stream = h->own_stream;
   cudaStream_t s = h->stream;
+
+  std::vector<Csc> mats;
+  if (h->sa()) {
+    // smoothed aggregation always uses the host setup; n_levels is a cap
+    sa_hierarchy(csc_from_arrays(n_rows, n_cols, colptr, rowidx, val), o.strength, o.n_levels, mats, h->sa_P);
+    h->L = (int)mats.size();
+  }
   const int L = h->L;
 
   // ---- level sizes (multigrid.hpp:127-130, :213-215) ----
@@ -2887,6 +2942,10 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
   h->n[0] = n_rows;
   if (h->bilinear()) h->m.assign(1, grid_lines(n_rows));
   for (int l = 1; l < L; ++l) {
+    if (h->sa()) {
+      h->n[l] = mats[l].cols;
+      continue;
+    }
     if (h->bilinear()) {
       h->m.push_back(coarse_lines_2d(h->m[l - 1]));
       h->n[l] = h->m[l] * h->m[l];
@@ -2902,12 +2961,11 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
   // Everything else (Gauss-Seidel schedules and colourings need the host matrices; unstructured
   // operators need SELL): host setup, every rank builds all of it.  AMGB_HOST_SETUP=1 forces the latter.
   std::vector<FullLevel> full;
-  std::vector<Csc> mats;
   const char* force_host = std::getenv("AMGB_HOST_SETUP");
-  if ((o.smoother == AMGB_SMOOTHER_JACOBI || o.smoother == AMGB_SMOOTHER_LINE_GS) &&
+  if ((o.smoother == AMGB_SMOOTHER_JACOBI || o.smoother == AMGB_SMOOTHER_LINE_GS) && !h->sa() &&
       !(force_host && std::string(force_host) == "1"))
     h->device_setup = device_build_levels(h.get(), n_rows, colptr, rowidx, val, full);
-  if (!h->device_setup) {
+  if (!h->device_setup && !h->sa()) {
     full.clear();
     h->raw_colptr.release();
     h->raw_rowidx.release();
@@ -3039,7 +3097,8 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
     S.u.zero(s);
     S.f.alloc(S.n_mat + 8);
     S.f.zero(s);
-    if (o.smoother == AMGB_SMOOTHER_JACOBI || S.sharded) {  // (sharded: every level vector is exported to the neighbours)
+    // (sharded: every level vector is exported to the neighbours; smoothed aggregation: the residual goes there)
+    if (o.smoother == AMGB_SMOOTHER_JACOBI || S.sharded || h->sa()) {
       S.tmp.alloc(S.n_vec() + 8);
       S.tmp.zero(s);
     }
@@ -3050,6 +3109,14 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
       if (want_window && !h->device_setup) h->ops[l]->build_window((int)(S.s - S.halo_lo), (int)S.n_vec(), s);
     }
     if (!(l + 1 == L && o.skip_dead_coarse_smooth)) h->prepare_smoother(l);
+  }
+  h->sa_R_rows.reserve(L);
+  h->sa_P_rows.reserve(L);
+  for (int l = 0; l + 1 < L && h->sa(); ++l) {
+    h->sa_R_rows.emplace_back();
+    h->sa_R_rows.back().upload(build_sell(h->sa_P[l]), s);
+    h->sa_P_rows.emplace_back();
+    h->sa_P_rows.back().upload(build_sell(transpose(h->sa_P[l])), s);
   }
   for (int l = 0; l < L; ++l) h->prepare_legs(l);
   {
@@ -3218,6 +3285,18 @@ int amgb_hierarchy_set_stream(amgb_hierarchy* h, void* cuda_stream) {
 }
 int amgb_hierarchy_n_levels(const amgb_hierarchy* h) { return h ? h->L : 0; }
 int amgb_hierarchy_transfer(const amgb_hierarchy* h) { return h ? h->opt.transfer : -1; }
+int amgb_hierarchy_get_transfer(const amgb_hierarchy* h, int level, int64_t* nnz, int* P_colptr, int* P_rowidx,
+                                double* P_val) {
+  return guarded([&] {
+    if (!h || !nnz) throw std::invalid_argument("null argument");
+    h->check_level(level, true);
+    const Csc P = h->prolongation(level);
+    *nnz = P.nnz();
+    if (P_colptr) std::memcpy(P_colptr, P.colptr.data(), P.colptr.size() * sizeof(int));
+    if (P_rowidx) std::memcpy(P_rowidx, P.rowidx.data(), P.rowidx.size() * sizeof(int));
+    if (P_val) std::memcpy(P_val, P.val.data(), P.val.size() * sizeof(double));
+  });
+}
 int64_t amgb_hierarchy_n_dofs(const amgb_hierarchy* h, int level) {
   return (h && level >= 0 && level < h->L) ? h->n[level] : -1;
 }
@@ -3476,7 +3555,9 @@ int amgb_restrict(amgb_hierarchy* h, int level, const double* r_fine, double* f_
     DevBuf<double> r, fc;
     r.upload(r_fine, h->n[level], h->stream);
     fc.alloc(h->n[level + 1]);
-    if (h->bilinear())
+    if (h->sa())
+      h->restrict_sa(r.p, fc.p, nullptr, level, h->stream);
+    else if (h->bilinear())
       h->restrict2d(r.p, fc.p, level, h->stream);
     else
       LAUNCH(dev::k_restrict, blocks_for(h->n[level + 1], 256), 256, 0, h->stream, r.p, (int)h->n[level],
@@ -3494,7 +3575,9 @@ int amgb_prolong_add(amgb_hierarchy* h, int level, const double* e_coarse, doubl
     DevBuf<double> e, uf;
     e.upload(e_coarse, h->n[level + 1], h->stream);
     uf.upload(u_fine, h->n[level], h->stream);
-    if (h->bilinear())
+    if (h->sa())
+      h->prolong_add_sa(e.p, uf.p, level, h->stream);
+    else if (h->bilinear())
       h->prolong_add2d(e.p, uf.p, level, h->stream);
     else
       LAUNCH(dev::k_prolong_add, blocks_for(h->n[level], 256), 256, 0, h->stream, e.p, 0, (int)h->n[level + 1],
@@ -3608,6 +3691,7 @@ int amgb_hierarchy_galerkin_device(amgb_hierarchy* h, int level, double* ms_out,
     CUDA_CHECK(cudaSetDevice(h->device));
     const DevMat& F = h->ops[level]->rows_of_A();
     const DevMat& Cm = h->ops[level + 1]->rows_of_A();
+    if (h->sa()) throw ApiError(AMGB_ESTATE, "the device-side Galerkin product covers the grid transfers only");
     if (!F.is_dia || !Cm.is_dia || F.dia.rows.p || Cm.dia.rows.p)
       throw ApiError(AMGB_ESTATE, "the device-side Galerkin product needs the DIA layout");
     gal::FineDia A;
@@ -3733,7 +3817,11 @@ int64_t amgb_hierarchy_vcycle_bytes(const amgb_hierarchy* h) {
       h->opt.smoother == AMGB_SMOOTHER_JACOBI ? h->opt.smoother_iters : 2 * h->opt.smoother_iters;
   for (int l = 0; l + 1 < h->L; ++l) {
     const int64_t B = amgb_hierarchy_pass_bytes(h, l);
-    total += (2 * passes_per_smooth + 1) * B + 24 * h->n[l] + 16 * h->n[l + 1];
+    total += (2 * passes_per_smooth + 1) * B;
+    if (h->sa())  // k_restrict_sa and k_prolong_add_sa stream R and P (12 B per entry each) besides the vectors
+      total += 12 * (h->sa_R_rows[l].nnz + h->sa_P_rows[l].nnz) + 24 * h->n[l] + 24 * h->n[l + 1];
+    else
+      total += 24 * h->n[l] + 16 * h->n[l + 1];
   }
   return total;
 }
@@ -3906,14 +3994,18 @@ int amgb_time_kernel(amgb_hierarchy* h, int level, int kind, int warmup, int rep
           A.residual(su, S.f.p, S.tmp_own(), s);
           break;
         case 2:
-          if (h->bilinear())
+          if (h->sa())  // the restriction alone: its residual is a separate k_residual launch (kind 1)
+            h->restrict_sa(scratch_u.p, scratch_c2.p, scratch_c.p, level, s);
+          else if (h->bilinear())
             A.residual_restrict2d(scratch_u.p, S.f.p, (int)h->m[level], 0, scratch_c2.p, scratch_c.p, (int)h->m[level + 1],
                                   0, 0, (int)h->m[level + 1], s);
           else
             A.residual_restrict(scratch_u.p, S.f.p, scratch_c2.p, scratch_c.p, (int)h->n[level + 1], s);
           break;
         case 3:
-          if (h->bilinear())
+          if (h->sa())
+            h->prolong_add_sa(scratch_c.p, scratch_u.p, level, s);
+          else if (h->bilinear())
             h->prolong_add2d(scratch_c.p, scratch_u.p, level, s);
           else
             LAUNCH(dev::k_prolong_add2, blocks_for((h->n[level] + 1) / 2, 256), 256, 0, s, scratch_c.p, 0,

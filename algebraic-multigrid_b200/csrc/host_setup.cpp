@@ -171,6 +171,141 @@ int64_t grid_lines(int64_t n) {
   return m * m == n ? m : -1;
 }
 
+// ------------------------------------------------------- smoothed aggregation
+
+// a_ii of every row (row i = CSC column i); a zero or absent diagonal is rejected
+static std::vector<double> sa_diagonal(const Csc& A, int level) {
+  std::vector<double> d(A.cols, 0.0);
+  for (int i = 0; i < A.cols; ++i)
+    for (int p = A.colptr[i]; p < A.colptr[i + 1]; ++p)
+      if (A.rowidx[p] == i) d[i] = A.val[p];
+  for (int i = 0; i < A.cols; ++i)
+    if (d[i] == 0.0)
+      throw std::invalid_argument("smoothed aggregation: level " + std::to_string(level) +
+                                  " has a zero diagonal at row " + std::to_string(i));
+  return d;
+}
+
+int64_t sa_aggregate(const Csc& A, double theta, std::vector<int>& agg, int level) {
+  if (!(theta >= 0.0))
+    throw std::invalid_argument("smoothed aggregation: strength must be >= 0, got " + std::to_string(theta));
+  if (A.rows != A.cols) throw std::invalid_argument("smoothed aggregation: A must be square");
+  const int n = A.cols;
+  const std::vector<double> d = sa_diagonal(A, level);
+  // strong neighbours of row i, ascending: |a_ij| > theta * sqrt(|a_ii| * |a_jj|), j != i, a_ij != 0
+  std::vector<int> sptr(n + 1, 0), snb;
+  snb.reserve(A.nnz());
+  for (int i = 0; i < n; ++i) {
+    for (int p = A.colptr[i]; p < A.colptr[i + 1]; ++p) {
+      const int j = A.rowidx[p];
+      const double a = A.val[p];
+      if (j == i || a == 0.0) continue;
+      const double thr = theta * std::sqrt(std::fabs(d[i]) * std::fabs(d[j]));
+      if (std::fabs(a) > thr) snb.push_back(j);
+    }
+    sptr[i + 1] = static_cast<int>(snb.size());
+  }
+  agg.assign(n, -1);
+  int64_t count = 0;
+  for (int i = 0; i < n; ++i) {  // pass 1: i and all its strong neighbours free -> new aggregate
+    if (agg[i] >= 0) continue;
+    bool free_nbrs = true;
+    for (int p = sptr[i]; p < sptr[i + 1] && free_nbrs; ++p) free_nbrs = agg[snb[p]] < 0;
+    if (!free_nbrs) continue;
+    const int J = static_cast<int>(count++);
+    agg[i] = J;
+    for (int p = sptr[i]; p < sptr[i + 1]; ++p) agg[snb[p]] = J;
+  }
+  const std::vector<int> pass1 = agg;
+  for (int i = 0; i < n; ++i) {  // pass 2: join the pass-1 aggregate of the first such strong neighbour
+    if (agg[i] >= 0) continue;
+    for (int p = sptr[i]; p < sptr[i + 1]; ++p)
+      if (pass1[snb[p]] >= 0) {
+        agg[i] = pass1[snb[p]];
+        break;
+      }
+  }
+  for (int i = 0; i < n; ++i) {  // pass 3: new aggregate with the still free strong neighbours
+    if (agg[i] >= 0) continue;
+    const int J = static_cast<int>(count++);
+    agg[i] = J;
+    for (int p = sptr[i]; p < sptr[i + 1]; ++p)
+      if (agg[snb[p]] < 0) agg[snb[p]] = J;
+  }
+  return count;
+}
+
+Csc sa_prolongation(const Csc& A, const std::vector<int>& agg, int64_t n_agg, int level) {
+  const int n = A.cols;
+  const std::vector<double> d = sa_diagonal(A, level);
+  // Gershgorin bound of D^-1 A over the stored entries
+  double rho = 0.0;
+  for (int i = 0; i < n; ++i) {
+    double s = 0.0;
+    for (int p = A.colptr[i]; p < A.colptr[i + 1]; ++p) s += std::fabs(A.val[p]);
+    rho = std::max(rho, s / std::fabs(d[i]));
+  }
+  const double w = (4.0 / 3.0) / rho;
+  // rows of P, built as the CSC columns of R = P^T
+  Csc R;
+  R.rows = static_cast<int>(n_agg);
+  R.cols = n;
+  R.colptr.assign((size_t)n + 1, 0);
+  std::vector<int> slot(n_agg, -1), touched;
+  std::vector<double> sums;
+  for (int i = 0; i < n; ++i) {
+    touched.clear();
+    sums.clear();
+    for (int p = A.colptr[i]; p < A.colptr[i + 1]; ++p) {
+      const int J = agg[A.rowidx[p]];
+      if (slot[J] < 0) {
+        slot[J] = static_cast<int>(touched.size());
+        touched.push_back(J);
+        sums.push_back(0.0);
+      }
+      sums[slot[J]] += A.val[p];
+    }
+    const double c = w / d[i];
+    std::vector<int> order(touched.size());
+    for (size_t t = 0; t < order.size(); ++t) order[t] = static_cast<int>(t);
+    std::sort(order.begin(), order.end(), [&](int a, int b) { return touched[a] < touched[b]; });
+    for (int t : order) {
+      const int J = touched[t];
+      const double prod = c * sums[t];
+      R.rowidx.push_back(J);
+      R.val.push_back((J == agg[i] ? 1.0 : 0.0) - prod);
+    }
+    for (int J : touched) slot[J] = -1;
+    if (R.rowidx.size() > static_cast<size_t>(std::numeric_limits<int>::max()))
+      throw std::overflow_error("sa_prolongation: P exceeds int32 indexing");
+    R.colptr[i + 1] = static_cast<int>(R.rowidx.size());
+  }
+  return transpose(R);
+}
+
+void sa_hierarchy(Csc&& A, double theta, int n_levels, std::vector<Csc>& mats, std::vector<Csc>& P) {
+  mats.clear();
+  P.clear();
+  mats.push_back(std::move(A));
+  while (static_cast<int>(mats.size()) < n_levels && mats.back().cols > kSaMaxCoarse) {
+    const int l = static_cast<int>(mats.size()) - 1;
+    std::vector<int> agg;
+    const int64_t n_agg = sa_aggregate(mats[l], theta, agg, l);
+    if (n_agg >= mats[l].cols) {
+      // level 0 (a diagonal matrix, say) has no hierarchy at all; a coarse level whose couplings are all weak
+      // (the Galerkin levels turn dense a few hundred rows above the 200-row target on large problems)
+      // becomes the coarsest level
+      if (l == 0)
+        throw std::invalid_argument("smoothed aggregation: the aggregation of level 0 does not reduce it (" +
+                                    std::to_string(mats[l].cols) + " rows, " + std::to_string(n_agg) + " aggregates)");
+      break;
+    }
+    P.push_back(sa_prolongation(mats[l], agg, n_agg, l));
+    Csc AH = galerkin(transpose(P.back()), mats[l], P.back());
+    mats.push_back(std::move(AH));
+  }
+}
+
 Csc multiply(const Csc& L, const Csc& R) {
   if (L.cols != R.rows) throw std::invalid_argument("multiply: inner dimensions differ");
   Csc C;

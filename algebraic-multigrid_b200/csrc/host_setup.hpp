@@ -44,6 +44,18 @@ int64_t coarse_lines_2d(int64_t m_h);
 Csc make_prolongation_2d(int64_t m_h, int64_t m_H);
 // m with m * m == n, or -1
 int64_t grid_lines(int64_t n);
+// Smoothed aggregation (AMGB_TRANSFER_SMOOTHED_AGGREGATION, specification in include/amgb.h and
+// tests/oracle_sa.py).  Row i of A is CSC column i.  sa_aggregate fills agg (one aggregate id per row,
+// ids in creation order) and returns the number of aggregates; sa_prolongation returns the smoothed P
+// (A.cols x n_agg).  Both throw std::invalid_argument naming `level` (and the row) on a zero diagonal;
+// sa_aggregate also on a strength threshold below 0 or NaN.
+int64_t sa_aggregate(const Csc& A, double theta, std::vector<int>& agg, int level = 0);
+Csc sa_prolongation(const Csc& A, const std::vector<int>& agg, int64_t n_agg, int level = 0);
+// The levels: mats[0] = A, then P[l] and mats[l + 1] = R (A P) with R = P^T while l + 1 < n_levels and
+// level l has more than kSaMaxCoarse rows.  A coarse level whose aggregation does not reduce it ends the
+// hierarchy as its coarsest level; when level 0 does not reduce, std::invalid_argument.
+constexpr int kSaMaxCoarse = 200;
+void sa_hierarchy(Csc&& A, double theta, int n_levels, std::vector<Csc>& mats, std::vector<Csc>& P);
 // Eigen 3.4.0 conservative ColMajor product: entry (i,j) = sum over ascending k
 // of L(i,k)*R(k,j); numerical zeros kept; result columns sorted.
 Csc multiply(const Csc& L, const Csc& R);

@@ -5,6 +5,7 @@
 // reference (:52-68), and apply the STORED operators: matrix-free on the GPU when those are the
 // linear-interpolation operators, through the generic device SpMV otherwise.
 #pragma once
+#include <stdexcept>
 #include <vector>
 
 #include "compat.hpp"
@@ -80,6 +81,8 @@ class InterpolatorBase {
   // AMGB_TRANSFER_* of the device kernels that apply this interpolator's operators matrix-free
   // (-1: none, the GPU driver cannot run it)
   virtual int device_transfer() const { return -1; }
+  // strength threshold theta of AMGB_TRANSFER_SMOOTHED_AGGREGATION (the library default for the others)
+  virtual double device_strength() const { return 0.08; }
   // true when P is the reference's linear interpolation
   bool is_linear_interpolation() const { return device_transfer() == AMGB_TRANSFER_LINEAR; }
 
@@ -178,6 +181,29 @@ class BilinearInterpolator2D : public InterpolatorBase<EleType> {
     while ((m + 1) * (m + 1) <= (int64_t)n) ++m;
     return m * m == (int64_t)n ? m : -1;
   }
+};
+
+// Smoothed-aggregation coarsening (no reference counterpart; include/amgb.h,
+// AMGB_TRANSFER_SMOOTHED_AGGREGATION): aggregates of strongly coupled rows (threshold theta), P smoothed by
+// one damped-Jacobi step.  It needs no grid.  n_levels is a cap: the hierarchy coarsens while a level has
+// more than 200 rows, and stops at a coarse level whose aggregation does not reduce it.  The aggregation depends on A, so Multigrid builds the operators and fills the P and
+// R slots; make_operators, which only knows the sizes, throws std::logic_error.
+template <class EleType>
+class SmoothedAggregationInterpolator : public InterpolatorBase<EleType> {
+ public:
+  explicit SmoothedAggregationInterpolator(size_t n_levels, double theta = 0.08)
+      : InterpolatorBase<EleType>(n_levels), theta_(theta) {}
+
+  void make_operators(size_t, size_t, size_t) override {
+    throw std::logic_error("SmoothedAggregationInterpolator: the aggregation depends on A, so Multigrid builds "
+                           "the operators (make_operators cannot build them from the level sizes)");
+  }
+  int device_transfer() const override { return AMGB_TRANSFER_SMOOTHED_AGGREGATION; }
+  double strength() const { return theta_; }
+  double device_strength() const override { return theta_; }
+
+ private:
+  double theta_;
 };
 
 }  // namespace AMG

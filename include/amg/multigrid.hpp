@@ -62,10 +62,12 @@ class Multigrid {
         throw std::invalid_argument("the GPU driver needs a SparseGaussSeidel, DampedJacobi, LineGaussSeidel or "
                                     "MulticolorGaussSeidel smoother");
       if (!interpolator || interpolator->device_transfer() < 0)
-        throw std::invalid_argument("the GPU driver applies the operators of LinearInterpolator or "
-                                    "BilinearInterpolator2D matrix-free");
+        throw std::invalid_argument("the GPU driver applies the operators of LinearInterpolator, "
+                                    "BilinearInterpolator2D or SmoothedAggregationInterpolator");
     }
     if (interpolator && interpolator->device_transfer() >= 0) opt.transfer = interpolator->device_transfer();
+    const bool sa = opt.transfer == AMGB_TRANSFER_SMOOTHED_AGGREGATION;
+    if (sa) opt.strength = interpolator->device_strength();
     if (smoother && smoother->device_kind() >= 0) {
       opt.smoother = smoother->device_kind();
       opt.smoother_iters = (int64_t)smoother->n_iters;
@@ -75,12 +77,15 @@ class Multigrid {
     if (!A.isCompressed()) throw std::invalid_argument("A must be compressed (makeCompressed())");
     detail::check(amgb_hierarchy_create((int)A.rows(), (int)A.cols(), A.outerIndexPtr(), A.innerIndexPtr(),
                                         A.valuePtr(), b.data(), (int64_t)b.rows(), &opt, &h));
+    n_levels = (size_t)amgb_hierarchy_n_levels(h);  // smoothed aggregation: n_levels_ is a cap
     level_to_coefficient_matrix.resize(n_levels);
     level_to_soln.resize(n_levels);
     level_to_rhs.resize(n_levels);
     // fill the interpolator's slots 0..L-2 like the reference's constructor does (:211-218)
-    for (size_t level = 1; level < n_levels; ++level)
-      interpolator->make_operators(get_n_dofs(level - 1), get_n_dofs(level), level - 1);
+    for (size_t level = 1; level < n_levels; ++level) {
+      if (sa) fill_transfer(level - 1);
+      else interpolator->make_operators(get_n_dofs(level - 1), get_n_dofs(level), level - 1);
+    }
   }
 
   void vcycle() { detail::check(amgb_vcycle(h)); }  // multigrid.hpp:263-305
@@ -159,6 +164,38 @@ class Multigrid {
     return get_soln(0);
   }
   amgb_hierarchy* handle() { return h; }
+  size_t get_n_levels() const { return n_levels; }
+
+ private:
+  // P of `level` as the hierarchy built it, and R = P^T (an index permutation), into the interpolator
+  void fill_transfer(size_t level) {
+    const int nf = (int)get_n_dofs(level), nc = (int)get_n_dofs(level + 1);
+    int64_t nnz = 0;
+    detail::check(amgb_hierarchy_get_transfer(h, (int)level, &nnz, nullptr, nullptr, nullptr));
+    std::vector<int> Pc(nc + 1), Pr(nnz), Rc(nf + 1, 0), Rr(nnz);
+    std::vector<double> Pv(nnz), Rv(nnz);
+    detail::check(amgb_hierarchy_get_transfer(h, (int)level, &nnz, Pc.data(), Pr.data(), Pv.data()));
+    for (int64_t p = 0; p < nnz; ++p) Rc[Pr[p] + 1]++;
+    for (int i = 0; i < nf; ++i) Rc[i + 1] += Rc[i];
+    std::vector<int> cursor(Rc.begin(), Rc.end() - 1);
+    for (int J = 0; J < nc; ++J)
+      for (int p = Pc[J]; p < Pc[J + 1]; ++p) {
+        const int q = cursor[Pr[p]]++;
+        Rr[q] = J;
+        Rv[q] = Pv[p];
+      }
+#if AMGB_HAVE_EIGEN
+    SparseMatrixT<EleType> P = Eigen::Map<const Eigen::SparseMatrix<double>>(nf, nc, nnz, Pc.data(), Pr.data(),
+                                                                             Pv.data());
+    SparseMatrixT<EleType> R = Eigen::Map<const Eigen::SparseMatrix<double>>(nc, nf, nnz, Rc.data(), Rr.data(),
+                                                                             Rv.data());
+#else
+    SparseMatrixT<EleType> P(nf, nc, std::move(Pc), std::move(Pr), std::move(Pv));
+    SparseMatrixT<EleType> R(nc, nf, std::move(Rc), std::move(Rr), std::move(Rv));
+#endif
+    interpolator->set_level_to_P(level, P);
+    interpolator->set_level_to_R(level, R);
+  }
 };
 
 }  // namespace AMG
