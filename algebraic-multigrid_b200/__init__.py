@@ -79,6 +79,7 @@ SIGNATURES = {
     "amgb_linear_restrict": (_i, [_l, _l, _pd, _pd]),
     "amgb_linear_prolong": (_i, [_l, _l, _pd, _pd]),
     "amgb_csc_spmv": (_i, [_i, _i, _pi, _pi, _pd, _pd, _pd]),
+    "amgb_csc_multiply": (_i, [_i, _i, _pi, _pi, _pd, _i, _pi, _pi, _pd, C.POINTER(_l), _p, _p, _p]),
     "amgb_matrix_create": (_i, [_i, _i, _pi, _pi, _pd, C.POINTER(_p)]),
     "amgb_matrix_destroy": (_i, [_p]),
     "amgb_matrix_nnz_device": (_l, [_p]),
@@ -100,6 +101,8 @@ SIGNATURES = {
     "amgb_hierarchy_destroy": (_i, [_p]),
     "amgb_hierarchy_transfer": (_i, [_p]),
     "amgb_hierarchy_get_transfer": (_i, [_p, _i, C.POINTER(_l), _p, _p, _p]),
+    "amgb_hierarchy_device_setup": (_i, [_p]),
+    "amgb_hierarchy_setup_times": (_i, [_p, _pd]),
     "amgb_comm_unique_id_bytes": (_i, []),
     "amgb_comm_get_unique_id": (_i, [_p]),
     "amgb_comm_create": (_i, [_p, _i, _i, C.POINTER(_p)]),
@@ -346,13 +349,27 @@ def sa_aggregate(A, strength=0.08):
     return agg, k.value
 
 
+def csc_multiply(A, B):
+    """A @ B of two CscMatrix on the device, in the order of the smoothed-aggregation setup's products: each
+    entry sums over ascending inner index, the first term initialising the sum; structural and computed
+    zeros are kept and every column comes out sorted."""
+    if A.cols != B.rows:
+        raise InvalidArgument(EINVAL, "csc_multiply: inner dimensions differ (%d x %d times %d x %d)"
+                              % (A.rows, A.cols, B.rows, B.cols))
+    nnz = _l()
+    args = (A.rows, A.cols, A.colptr, A.rowidx, A.val, B.cols, B.colptr, B.rowidx, B.val, C.byref(nnz))
+    _check(lib().amgb_csc_multiply(*args, None, None, None))
+    colptr, rowidx, val = np.empty(B.cols + 1, np.int32), np.empty(nnz.value, np.int32), np.empty(nnz.value)
+    _check(lib().amgb_csc_multiply(*args, colptr.ctypes.data, rowidx.ctypes.data, val.ctypes.data))
+    return CscMatrix(A.rows, B.cols, colptr, rowidx, val)
+
+
 def _transpose(M):
-    """CSC of M^T (an index permutation: entries keep their values, rows stay ascending)."""
-    order = np.argsort(M.rowidx, kind="stable")
-    colptr = np.zeros(M.rows + 1, np.int64)
-    np.add.at(colptr, M.rowidx.astype(np.int64) + 1, 1)
-    cols = np.repeat(np.arange(M.cols, dtype=np.int32), np.diff(M.colptr))
-    return CscMatrix(M.cols, M.rows, np.cumsum(colptr), cols[order], M.val[order])
+    """CSC of M^T (an index permutation: entries keep their values, rows stay ascending).  scipy's CSC -> CSR
+    conversion is a stable counting sort, linear in the entries."""
+    import scipy.sparse as sp
+    T = sp.csc_matrix((M.val, M.rowidx, M.colptr), shape=(M.rows, M.cols)).tocsr()
+    return CscMatrix(M.cols, M.rows, T.indptr, T.indices, T.data)
 
 
 class DeviceMatrix:
@@ -660,6 +677,18 @@ class Multigrid:
         _check(lib().amgb_hierarchy_get_transfer(self.h, level, C.byref(nnz), colptr.ctypes.data,
                                                  rowidx.ctypes.data, val.ctypes.data))
         return CscMatrix(nf, nc, colptr, rowidx, val)
+
+    @property
+    def device_setup(self):
+        """True when the level operators were built on the GPU (AMGB_HOST_SETUP=1 forces the host setup)."""
+        return bool(lib().amgb_hierarchy_device_setup(self.h))
+
+    def setup_times(self):
+        """Seconds of the setup phases of a smoothed-aggregation hierarchy (host clock, each phase ending in a
+        stream synchronise)."""
+        out = np.zeros(4)
+        _check(lib().amgb_hierarchy_setup_times(self.h, out))
+        return dict(zip(("aggregation", "prolongators", "galerkin", "mirrors"), out.tolist()))
 
     def get_tolerance(self):
         return lib().amgb_hierarchy_tolerance(self.h)

@@ -4,16 +4,22 @@
 // graph.  There is no CPU fallback: every compute entry point needs a device.
 #include "../../include/amgb.h"
 
+#include <algorithm>
 #include <atomic>
+#include <chrono>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <memory>
 #include <stdexcept>
 #include <string>
 #include <vector>
 
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
+#include <cub/device/device_segmented_sort.cuh>
 #include <cuda_runtime.h>
 
 #include "host_setup.hpp"
@@ -25,6 +31,7 @@
 #include "line_gs.cuh"
 #include "mid_levels.cuh"
 #include "setup_dia.cuh"
+#include "setup_sa.cuh"
 #include "transfer_sa.cuh"
 #include "stream_leg_api.hpp"
 #include "nccl_dyn.hpp"
@@ -223,6 +230,40 @@ struct DevMat {
                   : (int64_t)sell.val.n * 12 + (int64_t)sell.slice_ptr.n * 4 + (int64_t)sell.rows.n * 4;
   }
 };
+// A CSC matrix on the device (explicit zeros kept): the levels and prolongators of the device-side
+// smoothed-aggregation setup (setup_sa.cuh)
+struct DevCsc {
+  int rows = 0, cols = 0;
+  int64_t nnz = 0;
+  DevBuf<int> colptr, rowidx;
+  DevBuf<double> val;
+  sasetup::CscView view() const { return sasetup::CscView{rows, cols, colptr.p, rowidx.p, val.p}; }
+  void upload(int r, int c, const int* cp, const int* ri, const double* v, cudaStream_t s) {
+    rows = r;
+    cols = c;
+    nnz = cp[c];
+    colptr.upload(cp, (size_t)c + 1, s);
+    rowidx.upload(ri, (size_t)nnz, s);
+    val.upload(v, (size_t)nnz, s);
+    CUDA_CHECK(cudaStreamSynchronize(s));
+  }
+  Csc download(cudaStream_t s) const {
+    Csc M;
+    M.rows = rows;
+    M.cols = cols;
+    M.colptr.resize((size_t)cols + 1);
+    M.rowidx.resize((size_t)nnz);
+    M.val.resize((size_t)nnz);
+    CUDA_CHECK(cudaMemcpyAsync(M.colptr.data(), colptr.p, M.colptr.size() * sizeof(int), cudaMemcpyDeviceToHost, s));
+    if (nnz) {
+      CUDA_CHECK(cudaMemcpyAsync(M.rowidx.data(), rowidx.p, nnz * sizeof(int), cudaMemcpyDeviceToHost, s));
+      CUDA_CHECK(cudaMemcpyAsync(M.val.data(), val.p, nnz * sizeof(double), cudaMemcpyDeviceToHost, s));
+    }
+    CUDA_CHECK(cudaStreamSynchronize(s));
+    return M;
+  }
+};
+
 template <int ND>
 dev::DiaViewT<ND> dia_view_t(const DevDia& d) {
   dev::DiaViewT<ND> v;
@@ -328,6 +369,12 @@ struct Operator {
     n_mat = rowsA.n_rows;
     colrows.is_dia = true;
     colrows.dia = std::move(rowsA);
+  }
+  // the same with a rows-of-A mirror of either layout (device-side smoothed-aggregation setup)
+  void adopt_rows(DevMat&& rowsA) {
+    rows_primary = true;
+    n = n_mat = rowsA.n_rows();
+    colrows = std::move(rowsA);
   }
   const DevMat& rows_of_A() const { return (symmetric || block || rows_primary) ? colrows : *arows; }
   const Csc& host_rows_of_A() const { return symmetric ? M : MT; }  // CSC whose column k = row k of A
@@ -947,6 +994,12 @@ struct amgb_hierarchy {
   // of P_l) and the rows of P_l, both SELL-32
   std::vector<Csc> sa_P;
   std::vector<DevSell> sa_R_rows, sa_P_rows;
+  // device-side setup with the damped-Jacobi smoother: the level operators and P_l stay on the device as
+  // structural CSC (explicit zeros kept); the getters download them on demand into host_mats / a copy
+  bool sa_resident = false;
+  std::vector<DevCsc> sa_dev_A, sa_dev_P;
+  // seconds of [strength + aggregation, prolongators, Galerkin products, mirrors + coarsest factor]
+  double sa_times[4] = {0.0, 0.0, 0.0, 0.0};
   std::vector<std::unique_ptr<Operator>> ops;
   std::vector<LevelState> lv;
   DevBuf<double> partial, scalar;
@@ -1506,7 +1559,7 @@ struct amgb_hierarchy {
   }
   // P_l of this hierarchy's transfer kind (host setup)
   Csc prolongation(int l) const {
-    if (sa()) return sa_P[l];
+    if (sa()) return sa_resident ? sa_dev_P[l].download(stream) : sa_P[l];
     return bilinear() ? make_prolongation_2d(m[l], m[l + 1]) : make_prolongation(n[l], n[l + 1]);
   }
   void coarse_solve(cudaStream_t s) {  // multigrid.hpp:287-288
@@ -2205,7 +2258,12 @@ struct amgb_hierarchy {
   DevBuf<double> raw_val;
   std::vector<Csc> host_mats;
   const Csc& host_matrix(int level) {
-    if (!device_setup) return ops[level]->M;
+    if (sa_resident) {
+      if (host_mats.empty()) host_mats.resize(L);
+      if (host_mats[level].colptr.empty()) host_mats[level] = sa_dev_A[level].download(stream);
+      return host_mats[level];
+    }
+    if (!device_setup || sa()) return ops[level]->M;
     if (host_mats.empty()) {
       host_mats.resize(1);
       Csc& A = host_mats[0];
@@ -2743,6 +2801,327 @@ static void slice_level(const FullLevel& F, int n_src, int row_begin, int n_dst,
     }
   }
 }
+// ---- device-side smoothed-aggregation setup (setup_sa.cuh) ----
+// Exclusive prefix sum of c[0..n) into out[0..n] (out[n] = total), returned.
+static int64_t exclusive_scan(const long long* c, int64_t n, DevBuf<long long>& out, cudaStream_t s) {
+  out.alloc((size_t)n + 1);
+  out.zero(s);
+  if (n > 0) {
+    size_t bytes = 0;
+    CUDA_CHECK(cub::DeviceScan::InclusiveSum(nullptr, bytes, c, out.p + 1, n, s));
+    DevBuf<unsigned char> tmp;
+    tmp.alloc(bytes);
+    CUDA_CHECK(cub::DeviceScan::InclusiveSum(tmp.p, bytes, c, out.p + 1, n, s));
+  }
+  long long total = 0;
+  CUDA_CHECK(cudaMemcpyAsync(&total, out.p + n, sizeof(long long), cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaStreamSynchronize(s));
+  return total;
+}
+// int32 column pointers from the entry counts of n columns; overflow_error(what) beyond int32 indexing
+static int64_t counts_to_colptr(const long long* c, int64_t n, DevBuf<int>& colptr, const char* what, cudaStream_t s) {
+  DevBuf<long long> off;
+  const int64_t total = exclusive_scan(c, n, off, s);
+  if (total > (int64_t)std::numeric_limits<int>::max()) throw std::overflow_error(what);
+  colptr.alloc((size_t)n + 1);
+  LAUNCH(sasetup::k_narrow<int>, blocks_for(n + 1, 256), 256, 0, s, off.p, colptr.p, n + 1);
+  return total;
+}
+
+// T = A^T, entries of a column in ascending row (a stable sort of the entries by row; host: transpose)
+static void dev_transpose(const DevCsc& A, DevCsc& T, cudaStream_t s) {
+  const int64_t nnz = A.nnz;
+  T.rows = A.cols;
+  T.cols = A.rows;
+  T.nnz = nnz;
+  DevBuf<long long> counts;
+  counts.alloc((size_t)A.rows + 1);
+  counts.zero(s);
+  T.rowidx.alloc(nnz);
+  T.val.alloc(nnz);
+  if (nnz > 0) {
+    DevBuf<int> col_of, perm_in, perm, keys;
+    col_of.alloc(nnz);
+    perm_in.alloc(nnz);
+    perm.alloc(nnz);
+    keys.alloc(nnz);
+    LAUNCH(sasetup::k_col_of, blocks_for(A.cols, 256), 256, 0, s, A.colptr.p, A.cols, col_of.p);
+    LAUNCH(sasetup::k_iota, blocks_for(nnz, 256), 256, 0, s, perm_in.p, nnz);
+    LAUNCH(sasetup::k_row_count, blocks_for(nnz, 256), 256, 0, s, A.rowidx.p, nnz, counts.p);
+    int end_bit = 1;
+    while (end_bit < 31 && (1ll << end_bit) < (long long)A.rows) ++end_bit;
+    size_t bytes = 0;
+    CUDA_CHECK(cub::DeviceRadixSort::SortPairs(nullptr, bytes, A.rowidx.p, keys.p, perm_in.p, perm.p, (int)nnz, 0,
+                                               end_bit, s));
+    DevBuf<unsigned char> tmp;
+    tmp.alloc(bytes);
+    CUDA_CHECK(cub::DeviceRadixSort::SortPairs(tmp.p, bytes, A.rowidx.p, keys.p, perm_in.p, perm.p, (int)nnz, 0, end_bit,
+                                               s));
+    LAUNCH(sasetup::k_transpose_gather, blocks_for(nnz, 256), 256, 0, s, perm.p, col_of.p, A.val.p, nnz, T.rowidx.p,
+           T.val.p);
+  }
+  counts_to_colptr(counts.p, A.rows, T.colptr, "transpose: exceeds int32 indexing", s);
+}
+
+// bitwise_equal on the device
+static bool dev_equal(const DevCsc& A, const DevCsc& B, cudaStream_t s) {
+  if (A.rows != B.rows || A.cols != B.cols || A.nnz != B.nnz) return false;
+  DevBuf<int> flag;
+  flag.alloc(1);
+  flag.zero(s);
+  LAUNCH(sasetup::k_bits_differ<int>, blocks_for(A.cols + 1, 256), 256, 0, s, A.colptr.p, B.colptr.p, A.cols + 1, flag.p);
+  if (A.nnz > 0) {
+    LAUNCH(sasetup::k_bits_differ<int>, blocks_for(A.nnz, 256), 256, 0, s, A.rowidx.p, B.rowidx.p, A.nnz, flag.p);
+    LAUNCH(sasetup::k_bits_differ<double>, blocks_for(A.nnz, 256), 256, 0, s, A.val.p, B.val.p, A.nnz, flag.p);
+  }
+  int differ = 0;
+  CUDA_CHECK(cudaMemcpyAsync(&differ, flag.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaStreamSynchronize(s));
+  return !differ;
+}
+
+// C = L R in Eigen's conservative order (host: multiply; plus_zero: the sums start from +0).  what: the
+// overflow_error message when C exceeds int32 indexing.
+static void dev_multiply(const DevCsc& L, const DevCsc& R, DevCsc& C, bool plus_zero, const char* what, cudaStream_t s) {
+  if (L.cols != R.rows) throw std::invalid_argument("multiply: inner dimensions differ");
+  const int n = R.cols;
+  C.rows = L.rows;
+  C.cols = n;
+  DevBuf<long long> bound, count;
+  DevBuf<int> big, n_big;
+  DevBuf<unsigned long long> max_big;
+  bound.alloc(n);
+  count.alloc(n);
+  big.alloc(n);
+  n_big.alloc(1);
+  n_big.zero(s);
+  max_big.alloc(1);
+  max_big.zero(s);
+  if (n > 0)
+    LAUNCH(sasetup::k_spgemm_bound, blocks_for(n, 256), 256, 0, s, L.view(), R.view(), bound.p,
+           (long long)sasetup::kSmallSlots / 2, big.p, n_big.p, max_big.p);
+  int hb = 0;
+  unsigned long long hmax = 0;
+  CUDA_CHECK(cudaMemcpyAsync(&hb, n_big.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaMemcpyAsync(&hmax, max_big.p, sizeof(hmax), cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaStreamSynchronize(s));
+  // columns whose table exceeds the shared slots: per-warp tables in global memory, at most ~1 GB of them
+  int g_slots = 32;
+  while ((unsigned long long)g_slots < 2 * hmax) g_slots <<= 1;
+  const int64_t slot_bytes = (int64_t)g_slots * (sizeof(int) + sizeof(double));
+  const int64_t g_warps = std::max<int64_t>(1, std::min<int64_t>(hb, (1ll << 30) / slot_bytes));
+  const int g_blocks = blocks_for(g_warps, sasetup::kSpgemmWarps);
+  DevBuf<int> g_keys;
+  DevBuf<double> g_vals;
+  if (hb > 0) {
+    g_keys.alloc((size_t)g_blocks * sasetup::kSpgemmWarps * g_slots);
+    g_vals.alloc((size_t)g_blocks * sasetup::kSpgemmWarps * g_slots);
+  }
+  const int threads = sasetup::kSpgemmWarps * 32;
+  const int s_blocks = std::max(1, std::min(blocks_for(n, sasetup::kSpgemmWarps), 8192));
+  auto run = [&](auto kern, int* c_rowidx, double* c_val, const long long* cptr) {
+    CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sasetup::kSpgemmSmem));
+    if (n > 0)
+      LAUNCH(kern, s_blocks, threads, sasetup::kSpgemmSmem, s, L.view(), R.view(), bound.p, nullptr, 0, nullptr,
+             nullptr, 0, count.p, cptr, c_rowidx, c_val);
+    if (hb > 0)
+      LAUNCH(kern, g_blocks, threads, 0, s, L.view(), R.view(), bound.p, big.p, hb, g_keys.p, g_vals.p, g_slots,
+             count.p, cptr, c_rowidx, c_val);
+  };
+  // symbolic pass: entries per column
+  run(sasetup::k_spgemm<false, false>, nullptr, nullptr, nullptr);
+  DevBuf<long long> off;
+  const int64_t total = exclusive_scan(count.p, n, off, s);
+  if (total > (int64_t)std::numeric_limits<int>::max()) throw std::overflow_error(what);
+  C.nnz = total;
+  C.colptr.alloc((size_t)n + 1);
+  LAUNCH(sasetup::k_narrow<int>, blocks_for((int64_t)n + 1, 256), 256, 0, s, off.p, C.colptr.p, (int64_t)n + 1);
+  // numeric pass (unsorted columns), then every column sorted by row
+  DevBuf<int> rowidx_u;
+  DevBuf<double> val_u;
+  rowidx_u.alloc(total);
+  val_u.alloc(total);
+  if (plus_zero) run(sasetup::k_spgemm<true, true>, rowidx_u.p, val_u.p, off.p);
+  else run(sasetup::k_spgemm<true, false>, rowidx_u.p, val_u.p, off.p);
+  C.rowidx.alloc(total);
+  C.val.alloc(total);
+  if (total > 0) {
+    size_t bytes = 0;
+    CUDA_CHECK(cub::DeviceSegmentedSort::SortPairs(nullptr, bytes, rowidx_u.p, C.rowidx.p, val_u.p, C.val.p, (int)total,
+                                                   n, C.colptr.p, C.colptr.p + 1, s));
+    DevBuf<unsigned char> tmp;
+    tmp.alloc(bytes);
+    CUDA_CHECK(cub::DeviceSegmentedSort::SortPairs(tmp.p, bytes, rowidx_u.p, C.rowidx.p, val_u.p, C.val.p, (int)total, n,
+                                                   C.colptr.p, C.colptr.p + 1, s));
+  }
+  CUDA_CHECK(cudaStreamSynchronize(s));
+}
+
+// build_sell of a device CSC ("row c = CSC column c", explicit zeros dropped), on the device
+static void dev_sell(const DevCsc& M, DevSell& S, cudaStream_t s) {
+  const int n = M.cols;
+  const int n_slices = (n + 31) / 32;
+  DevBuf<int> len;
+  DevBuf<unsigned long long> nnz;
+  DevBuf<long long> size;
+  len.alloc(n);
+  nnz.alloc(1);
+  nnz.zero(s);
+  size.alloc(n_slices);
+  if (n > 0) {
+    LAUNCH(sasetup::k_sell_len, blocks_for(n, 256), 256, 0, s, M.view(), len.p, nnz.p);
+    LAUNCH(sasetup::k_sell_slice_size, blocks_for(n, 256), 256, 0, s, len.p, n, size.p);
+  }
+  DevBuf<long long> off;
+  const int64_t total = exclusive_scan(size.p, n_slices, off, s);
+  if (total > 0xffffffffll) throw std::overflow_error("SELL layout exceeds 32-bit offsets");
+  S.n_rows = n;
+  S.n_slices = n_slices;
+  S.slice_ptr.alloc((size_t)n_slices + 1);
+  LAUNCH(sasetup::k_narrow<uint32_t>, blocks_for((int64_t)n_slices + 1, 256), 256, 0, s, off.p, S.slice_ptr.p,
+         (int64_t)n_slices + 1);
+  S.col.alloc(total);
+  S.val.alloc(total);
+  CUDA_CHECK(cudaMemsetAsync(S.col.p, 0xff, std::max<int64_t>(total, 1) * sizeof(int), s));
+  S.val.zero(s);
+  S.rows.release();
+  if (n > 0) LAUNCH(sasetup::k_sell_fill, blocks_for(n, 256), 256, 0, s, M.view(), off.p, S.col.p, S.val.p);
+  unsigned long long hn = 0;
+  CUDA_CHECK(cudaMemcpyAsync(&hn, nnz.p, sizeof(hn), cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaStreamSynchronize(s));
+  S.nnz = (int64_t)hn;
+}
+
+// build_dia of a square device CSC on the device; false where build_dia refuses (more than 16 offsets, or
+// diagonal storage streaming > 25 % more bytes than SELL)
+static bool dev_dia(const DevCsc& M, DevDia& D, cudaStream_t s) {
+  const int n = M.cols;
+  if (n < 1 || M.rows != n) return false;
+  const int shift = n - 1;
+  const int n_words = (2 * n - 1 + 31) / 32;
+  DevBuf<unsigned> bitmap;
+  bitmap.alloc(n_words);
+  bitmap.zero(s);
+  DevBuf<int> list;
+  list.alloc(2 + setup::kMaxOffsets);
+  list.zero(s);
+  LAUNCH(sasetup::k_mark_offsets_nz, blocks_for(n, 256), 256, 0, s, M.view(), shift, bitmap.p);
+  LAUNCH(setup::k_collect_offsets, blocks_for(n_words, 256), 256, 0, s, bitmap.p, n_words, shift, setup::kMaxOffsets,
+         list.p);
+  std::vector<int> hl(2 + setup::kMaxOffsets, 0);
+  CUDA_CHECK(cudaMemcpyAsync(hl.data(), list.p, hl.size() * sizeof(int), cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaStreamSynchronize(s));
+  if (hl[0] < 1 || hl[0] > setup::kMaxOffsets) return false;
+  std::vector<int> off(hl.begin() + 1, hl.begin() + 1 + hl[0]);
+  std::sort(off.begin(), off.end());
+  setup::Offsets o{};
+  o.n = (int)off.size();
+  for (int d = 0; d < o.n; ++d) o.v[d] = off[d];
+  const int ld = (n + 31) / 32 * 32;
+  DevBuf<double> val;
+  val.alloc((size_t)off.size() * ld);
+  val.zero(s);
+  LAUNCH(sasetup::k_csc_to_dia_nz, blocks_for(n, 256), 256, 0, s, M.colptr.p, M.rowidx.p, M.val.p, n, o, val.p, ld);
+  FullLevel F;
+  if (!finalize_full_level(F, std::move(val), off, n, ld, s)) return false;
+  D = std::move(F.dia);
+  return true;
+}
+
+// DevMat::upload of a device CSC: DIA when build_dia accepts it, else SELL-32
+static void dev_mat(const DevCsc& M, DevMat& out, cudaStream_t s) {
+  out.is_dia = dev_dia(M, out.dia, s);
+  if (!out.is_dia) dev_sell(M, out.sell, s);
+}
+
+// sa_hierarchy on the device: A[0] = the level-0 operator, then P[l], R[l] = P[l]^T and A[l + 1] = R (A P)
+// while the hierarchy grows (same stop rule, same errors).  The strong graph of every level is downloaded
+// and aggregated on the host by the same passes as sa_aggregate.  phase_s accumulates the seconds of
+// [strength + aggregation, prolongators, Galerkin products], each phase ending in a stream synchronise.
+static void sa_device_hierarchy(int n_levels, double theta, std::vector<DevCsc>& A, std::vector<DevCsc>& P,
+                                std::vector<DevCsc>& R, double* phase_s, cudaStream_t s) {
+  using clock = std::chrono::steady_clock;
+  auto lap = [&](clock::time_point& t0, int phase) {
+    CUDA_CHECK(cudaStreamSynchronize(s));
+    const clock::time_point t1 = clock::now();
+    phase_s[phase] += std::chrono::duration<double>(t1 - t0).count();
+    t0 = t1;
+  };
+  P.clear();
+  R.clear();
+  while ((int)A.size() < n_levels && A.back().cols > kSaMaxCoarse) {
+    const int l = (int)A.size() - 1;
+    const int n = A[l].cols;
+    const sasetup::CscView M = A[l].view();
+    clock::time_point t0 = clock::now();
+    // diagonal and strength graph
+    DevBuf<double> d;
+    d.alloc(n);
+    DevBuf<int> zero_row;
+    const int none = std::numeric_limits<int>::max();
+    zero_row.upload(&none, 1, s);
+    LAUNCH(sasetup::k_sa_diag, blocks_for(n, 256), 256, 0, s, M, d.p, zero_row.p);
+    int zr = none;
+    CUDA_CHECK(cudaMemcpyAsync(&zr, zero_row.p, sizeof(int), cudaMemcpyDeviceToHost, s));
+    CUDA_CHECK(cudaStreamSynchronize(s));
+    if (zr != none) throw std::invalid_argument(sa_zero_diagonal_message(l, zr));
+    DevBuf<long long> cnt, sptr;
+    cnt.alloc(n);
+    LAUNCH(sasetup::k_sa_strength<false>, blocks_for(n, 256), 256, 0, s, M, d.p, theta, cnt.p, nullptr, nullptr);
+    const int64_t n_strong = exclusive_scan(cnt.p, n, sptr, s);
+    DevBuf<int> snb, sptr32;
+    snb.alloc(n_strong);
+    sptr32.alloc((size_t)n + 1);
+    LAUNCH(sasetup::k_sa_strength<true>, blocks_for(n, 256), 256, 0, s, M, d.p, theta, nullptr, sptr.p, snb.p);
+    LAUNCH(sasetup::k_narrow<int>, blocks_for((int64_t)n + 1, 256), 256, 0, s, sptr.p, sptr32.p, (int64_t)n + 1);
+    std::vector<int> h_sptr((size_t)n + 1), h_snb((size_t)n_strong);
+    sptr32.download(h_sptr.data(), s);
+    snb.download(h_snb.data(), s);
+    CUDA_CHECK(cudaStreamSynchronize(s));
+    std::vector<int> agg;
+    const int64_t n_agg = sa_aggregate_passes(n, h_sptr.data(), h_snb.data(), agg);
+    if (n_agg >= n) {
+      if (l == 0) throw std::invalid_argument(sa_no_reduction_message(n, n_agg));
+      break;
+    }
+    DevCsc T;  // aggregate indicator, transposed: column k holds (agg[k], 1.0)
+    T.rows = (int)n_agg;
+    T.cols = n;
+    T.nnz = n;
+    T.rowidx.upload(agg, s);
+    T.colptr.alloc((size_t)n + 1);
+    T.val.alloc(n);
+    LAUNCH(sasetup::k_iota, blocks_for((int64_t)n + 1, 256), 256, 0, s, T.colptr.p, (int64_t)n + 1);
+    LAUNCH(sasetup::k_fill, blocks_for(n, 256), 256, 0, s, T.val.p, n, 1.0);
+    lap(t0, 0);
+    // smoothed prolongator, built as R = P^T: S = T A sums the entries of every row i per aggregate, then
+    // R(J, i) = (J == agg[i]) - (w / a_ii) S(J, i)
+    DevBuf<unsigned long long> rho_bits;
+    rho_bits.alloc(1);
+    rho_bits.zero(s);
+    LAUNCH(sasetup::k_sa_gershgorin, blocks_for(n, 256), 256, 0, s, M, d.p, rho_bits.p);
+    unsigned long long rb = 0;
+    CUDA_CHECK(cudaMemcpyAsync(&rb, rho_bits.p, sizeof(rb), cudaMemcpyDeviceToHost, s));
+    CUDA_CHECK(cudaStreamSynchronize(s));
+    double rho;
+    std::memcpy(&rho, &rb, sizeof(rho));
+    const double w = (4.0 / 3.0) / rho;
+    DevCsc Rl, Pl;
+    dev_multiply(T, A[l], Rl, true, "sa_prolongation: P exceeds int32 indexing", s);
+    LAUNCH(sasetup::k_sa_smooth, blocks_for(n, 256), 256, 0, s, n, Rl.colptr.p, Rl.rowidx.p, Rl.val.p, T.rowidx.p, d.p, w);
+    dev_transpose(Rl, Pl, s);
+    lap(t0, 1);
+    // Galerkin product A_{l+1} = R (A P)
+    DevCsc AP, AH;
+    dev_multiply(A[l], Pl, AP, false, "multiply: result exceeds int32 indexing", s);
+    dev_multiply(Rl, AP, AH, false, "multiply: result exceeds int32 indexing", s);
+    lap(t0, 2);
+    P.push_back(std::move(Pl));
+    R.push_back(std::move(Rl));
+    A.push_back(std::move(AH));
+  }
+}
+
 // The whole hierarchy on the device: level 0 from the raw CSC arrays, levels >= 1 by Galerkin products.
 // false: the operator (or one of its coarse operators) does not fit the DIA layout -> host setup.
 static bool device_build_levels(amgb_hierarchy* h, int n_rows, const int* colptr, const int* rowidx, const double* val,
@@ -2930,10 +3309,52 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
   cudaStream_t s = h->stream;
 
   std::vector<Csc> mats;
+  const char* force_host = std::getenv("AMGB_HOST_SETUP");
+  const bool host_setup = force_host && std::string(force_host) == "1";
+  using clock = std::chrono::steady_clock;
+  clock::time_point sa_t0 = clock::now();
+  std::vector<DevMat> sa_rows;  // rows-of-A mirrors of a device-resident smoothed-aggregation hierarchy
   if (h->sa()) {
-    // smoothed aggregation always uses the host setup; n_levels is a cap
-    sa_hierarchy(csc_from_arrays(n_rows, n_cols, colptr, rowidx, val), o.strength, o.n_levels, mats, h->sa_P);
-    h->L = (int)mats.size();
+    // n_levels is a cap.  Device setup unless AMGB_HOST_SETUP=1: the levels and prolongators are built on
+    // the GPU; damped Jacobi keeps them there, the Gauss-Seidel smoothers (whose colourings and schedules
+    // need host matrices) download them and continue like the host setup
+    if (host_setup) {
+      sa_hierarchy(csc_from_arrays(n_rows, n_cols, colptr, rowidx, val), o.strength, o.n_levels, mats, h->sa_P,
+                   h->sa_times);
+      h->L = (int)mats.size();
+      sa_t0 = clock::now();
+    } else {
+      std::vector<DevCsc> A(1), R;
+      A[0].upload(n_rows, n_cols, colptr, rowidx, val, s);
+      sa_device_hierarchy(o.n_levels, o.strength, A, h->sa_dev_P, R, h->sa_times, s);
+      h->device_setup = true;
+      h->L = (int)A.size();
+      sa_t0 = clock::now();
+      const int L = h->L;
+      if (o.smoother == AMGB_SMOOTHER_JACOBI) {
+        h->sa_resident = true;
+        // mirrors: the rows of A (A itself when bitwise symmetric), and SELL rows of R and of P
+        sa_rows.resize(L);
+        for (int l = 0; l < L; ++l) {
+          DevCsc AT;
+          dev_transpose(A[l], AT, s);
+          dev_mat(dev_equal(A[l], AT, s) ? A[l] : AT, sa_rows[l], s);
+        }
+        for (int l = 0; l + 1 < L; ++l) {
+          h->sa_R_rows.emplace_back();
+          dev_sell(h->sa_dev_P[l], h->sa_R_rows.back(), s);
+          h->sa_P_rows.emplace_back();
+          dev_sell(R[l], h->sa_P_rows.back(), s);
+        }
+        mats.resize(L);
+        mats[L - 1] = A[L - 1].download(s);  // the coarsest factorisation and its size check
+        h->sa_dev_A = std::move(A);
+      } else {
+        for (const DevCsc& M : A) mats.push_back(M.download(s));
+        for (const DevCsc& M : h->sa_dev_P) h->sa_P.push_back(M.download(s));
+        h->sa_dev_P.clear();
+      }
+    }
   }
   const int L = h->L;
 
@@ -2943,7 +3364,7 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
   if (h->bilinear()) h->m.assign(1, grid_lines(n_rows));
   for (int l = 1; l < L; ++l) {
     if (h->sa()) {
-      h->n[l] = mats[l].cols;
+      h->n[l] = h->sa_resident ? h->sa_dev_A[l].cols : mats[l].cols;
       continue;
     }
     if (h->bilinear()) {
@@ -2961,10 +3382,9 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
   // Everything else (Gauss-Seidel schedules and colourings need the host matrices; unstructured
   // operators need SELL): host setup, every rank builds all of it.  AMGB_HOST_SETUP=1 forces the latter.
   std::vector<FullLevel> full;
-  const char* force_host = std::getenv("AMGB_HOST_SETUP");
-  if ((o.smoother == AMGB_SMOOTHER_JACOBI || o.smoother == AMGB_SMOOTHER_LINE_GS) && !h->sa() &&
-      !(force_host && std::string(force_host) == "1"))
+  if ((o.smoother == AMGB_SMOOTHER_JACOBI || o.smoother == AMGB_SMOOTHER_LINE_GS) && !h->sa() && !host_setup)
     h->device_setup = device_build_levels(h.get(), n_rows, colptr, rowidx, val, full);
+  const bool dia_setup = h->device_setup && !h->sa();  // levels built by device_build_levels
   if (!h->device_setup && !h->sa()) {
     full.clear();
     h->raw_colptr.release();
@@ -2983,7 +3403,7 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
   std::vector<std::vector<int>> level_off(L);
   std::vector<int> half_bw(L, 0);
   for (int l = 0; l < L; ++l) {
-    if (h->device_setup) {
+    if (dia_setup) {
       level_off[l] = full[l].off;
     } else {
       const Csc& M = mats[l];
@@ -3008,7 +3428,7 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
       throw std::invalid_argument("coarsest level too large for the direct solve (" + std::to_string(nc) +
                                   " DOF, half-bandwidth " + std::to_string(bw) + "): use more levels");
   }
-  h->factor = h->device_setup ? factor_banded_ldlt(csc_from_device_dia(full[L - 1].dia, s)) : factor_banded_ldlt(mats[L - 1]);
+  h->factor = dia_setup ? factor_banded_ldlt(csc_from_device_dia(full[L - 1].dia, s)) : factor_banded_ldlt(mats[L - 1]);
 
   // ---- partition (sharded runs only) ----
   const int world = comm ? comm->world : 1;
@@ -3067,7 +3487,7 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
       S.halo_hi = h->plan.halo_hi[l];
       S.n_own = (int)(S.e - S.s);
       S.n_mat = (int)std::min<int64_t>(S.n_own + h->plan.ghost[l], h->n[l] - S.s);
-      if (h->device_setup) {
+      if (dia_setup) {
         // row block (+ ghost rows) and window of this rank, sliced out of the whole level on the device
         DevDia blk;
         slice_level(full[l], (int)h->n[l], (int)S.s, S.n_mat, blk, true, s);
@@ -3089,7 +3509,8 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
       S.s = 0;
       S.e = h->n[l];
       S.n_own = S.n_mat = (int)h->n[l];
-      if (h->device_setup) h->ops[l]->adopt_rows(std::move(full[l].dia), S.n_own);
+      if (dia_setup) h->ops[l]->adopt_rows(std::move(full[l].dia), S.n_own);
+      else if (h->sa_resident) h->ops[l]->adopt_rows(std::move(sa_rows[l]));
       else h->ops[l]->build(std::move(mats[l]), s);
     }
     // +8: the fused legs copy 16-byte aligned windows, which may reach one entry past the end
@@ -3106,17 +3527,19 @@ static void create_hierarchy(amgb_comm* comm, int64_t min_rows_per_rank, int n_r
       S.fw.alloc(S.n_vec() + 8);
       S.fw.zero(s);
       // window mirror of the operator for the fused legs (block + ghost rows on both sides)
-      if (want_window && !h->device_setup) h->ops[l]->build_window((int)(S.s - S.halo_lo), (int)S.n_vec(), s);
+      if (want_window && !dia_setup) h->ops[l]->build_window((int)(S.s - S.halo_lo), (int)S.n_vec(), s);
     }
     if (!(l + 1 == L && o.skip_dead_coarse_smooth)) h->prepare_smoother(l);
   }
-  h->sa_R_rows.reserve(L);
-  h->sa_P_rows.reserve(L);
-  for (int l = 0; l + 1 < L && h->sa(); ++l) {
+  for (int l = 0; l + 1 < L && h->sa() && !h->sa_resident; ++l) {
     h->sa_R_rows.emplace_back();
     h->sa_R_rows.back().upload(build_sell(h->sa_P[l]), s);
     h->sa_P_rows.emplace_back();
     h->sa_P_rows.back().upload(build_sell(transpose(h->sa_P[l])), s);
+  }
+  if (h->sa()) {
+    CUDA_CHECK(cudaStreamSynchronize(s));
+    h->sa_times[3] = std::chrono::duration<double>(clock::now() - sa_t0).count();
   }
   for (int l = 0; l < L; ++l) h->prepare_legs(l);
   {
@@ -3297,12 +3720,44 @@ int amgb_hierarchy_get_transfer(const amgb_hierarchy* h, int level, int64_t* nnz
     if (P_val) std::memcpy(P_val, P.val.data(), P.val.size() * sizeof(double));
   });
 }
+// C = A B for host CSC matrices (A: m x k, B: k x n), computed on the device in Eigen's conservative order
+// (host_setup.cpp: multiply); the product of the smoothed-aggregation setup
+int amgb_csc_multiply(int m, int k, const int* A_colptr, const int* A_rowidx, const double* A_val, int n,
+                      const int* B_colptr, const int* B_rowidx, const double* B_val, int64_t* nnz, int* C_colptr,
+                      int* C_rowidx, double* C_val) {
+  return guarded([&] {
+    if (!nnz || !A_colptr || !B_colptr || m < 0 || k < 0 || n < 0) throw std::invalid_argument("bad multiply arguments");
+    if (A_colptr[k] > 0 && (!A_rowidx || !A_val)) throw std::invalid_argument("bad multiply arguments");
+    if (B_colptr[n] > 0 && (!B_rowidx || !B_val)) throw std::invalid_argument("bad multiply arguments");
+    require_device();
+    cudaStream_t s = nullptr;
+    DevCsc A, B, C;
+    A.upload(m, k, A_colptr, A_rowidx, A_val, s);
+    B.upload(k, n, B_colptr, B_rowidx, B_val, s);
+    dev_multiply(A, B, C, false, "multiply: result exceeds int32 indexing", s);
+    *nnz = C.nnz;
+    if (C_colptr) C.colptr.download(C_colptr, s);
+    if (C_rowidx) C.rowidx.download(C_rowidx, s);
+    if (C_val) C.val.download(C_val, s);
+    CUDA_CHECK(cudaStreamSynchronize(s));
+  });
+}
+
+int amgb_hierarchy_device_setup(const amgb_hierarchy* h) { return h && h->device_setup ? 1 : 0; }
+int amgb_hierarchy_setup_times(const amgb_hierarchy* h, double* out) {
+  return guarded([&] {
+    if (!h || !out) throw std::invalid_argument("null argument");
+    if (!h->sa()) throw ApiError(AMGB_ESTATE, "setup phase times are recorded for smoothed-aggregation hierarchies only");
+    for (int i = 0; i < 4; ++i) out[i] = h->sa_times[i];
+  });
+}
 int64_t amgb_hierarchy_n_dofs(const amgb_hierarchy* h, int level) {
   return (h && level >= 0 && level < h->L) ? h->n[level] : -1;
 }
 int64_t amgb_hierarchy_nnz(const amgb_hierarchy* h, int level) {
   if (!h || level < 0 || level >= h->L) return -1;
   try {
+    if (h->sa_resident) return h->sa_dev_A[level].nnz;
     return const_cast<amgb_hierarchy*>(h)->host_matrix(level).nnz();
   } catch (...) {
     return -1;

@@ -2,6 +2,7 @@
 #include "host_setup.hpp"
 
 #include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <cstring>
 #include <limits>
@@ -173,6 +174,15 @@ int64_t grid_lines(int64_t n) {
 
 // ------------------------------------------------------- smoothed aggregation
 
+std::string sa_zero_diagonal_message(int level, int row) {
+  return "smoothed aggregation: level " + std::to_string(level) + " has a zero diagonal at row " + std::to_string(row);
+}
+
+std::string sa_no_reduction_message(int rows, int64_t n_agg) {
+  return "smoothed aggregation: the aggregation of level 0 does not reduce it (" + std::to_string(rows) + " rows, " +
+         std::to_string(n_agg) + " aggregates)";
+}
+
 // a_ii of every row (row i = CSC column i); a zero or absent diagonal is rejected
 static std::vector<double> sa_diagonal(const Csc& A, int level) {
   std::vector<double> d(A.cols, 0.0);
@@ -180,20 +190,19 @@ static std::vector<double> sa_diagonal(const Csc& A, int level) {
     for (int p = A.colptr[i]; p < A.colptr[i + 1]; ++p)
       if (A.rowidx[p] == i) d[i] = A.val[p];
   for (int i = 0; i < A.cols; ++i)
-    if (d[i] == 0.0)
-      throw std::invalid_argument("smoothed aggregation: level " + std::to_string(level) +
-                                  " has a zero diagonal at row " + std::to_string(i));
+    if (d[i] == 0.0) throw std::invalid_argument(sa_zero_diagonal_message(level, i));
   return d;
 }
 
-int64_t sa_aggregate(const Csc& A, double theta, std::vector<int>& agg, int level) {
+void sa_strength(const Csc& A, double theta, std::vector<int>& sptr, std::vector<int>& snb, int level) {
   if (!(theta >= 0.0))
     throw std::invalid_argument("smoothed aggregation: strength must be >= 0, got " + std::to_string(theta));
   if (A.rows != A.cols) throw std::invalid_argument("smoothed aggregation: A must be square");
   const int n = A.cols;
   const std::vector<double> d = sa_diagonal(A, level);
   // strong neighbours of row i, ascending: |a_ij| > theta * sqrt(|a_ii| * |a_jj|), j != i, a_ij != 0
-  std::vector<int> sptr(n + 1, 0), snb;
+  sptr.assign((size_t)n + 1, 0);
+  snb.clear();
   snb.reserve(A.nnz());
   for (int i = 0; i < n; ++i) {
     for (int p = A.colptr[i]; p < A.colptr[i + 1]; ++p) {
@@ -205,6 +214,9 @@ int64_t sa_aggregate(const Csc& A, double theta, std::vector<int>& agg, int leve
     }
     sptr[i + 1] = static_cast<int>(snb.size());
   }
+}
+
+int64_t sa_aggregate_passes(int n, const int* sptr, const int* snb, std::vector<int>& agg) {
   agg.assign(n, -1);
   int64_t count = 0;
   for (int i = 0; i < n; ++i) {  // pass 1: i and all its strong neighbours free -> new aggregate
@@ -233,6 +245,12 @@ int64_t sa_aggregate(const Csc& A, double theta, std::vector<int>& agg, int leve
       if (agg[snb[p]] < 0) agg[snb[p]] = J;
   }
   return count;
+}
+
+int64_t sa_aggregate(const Csc& A, double theta, std::vector<int>& agg, int level) {
+  std::vector<int> sptr, snb;
+  sa_strength(A, theta, sptr, snb, level);
+  return sa_aggregate_passes(A.cols, sptr.data(), snb.data(), agg);
 }
 
 Csc sa_prolongation(const Csc& A, const std::vector<int>& agg, int64_t n_agg, int level) {
@@ -283,26 +301,35 @@ Csc sa_prolongation(const Csc& A, const std::vector<int>& agg, int64_t n_agg, in
   return transpose(R);
 }
 
-void sa_hierarchy(Csc&& A, double theta, int n_levels, std::vector<Csc>& mats, std::vector<Csc>& P) {
+void sa_hierarchy(Csc&& A, double theta, int n_levels, std::vector<Csc>& mats, std::vector<Csc>& P,
+                  double* phase_s) {
+  using clock = std::chrono::steady_clock;
+  auto lap = [&](clock::time_point& t0, int phase) {
+    const clock::time_point t1 = clock::now();
+    if (phase_s) phase_s[phase] += std::chrono::duration<double>(t1 - t0).count();
+    t0 = t1;
+  };
   mats.clear();
   P.clear();
   mats.push_back(std::move(A));
   while (static_cast<int>(mats.size()) < n_levels && mats.back().cols > kSaMaxCoarse) {
     const int l = static_cast<int>(mats.size()) - 1;
     std::vector<int> agg;
+    clock::time_point t0 = clock::now();
     const int64_t n_agg = sa_aggregate(mats[l], theta, agg, l);
+    lap(t0, 0);
     if (n_agg >= mats[l].cols) {
       // level 0 (a diagonal matrix, say) has no hierarchy at all; a coarse level whose couplings are all weak
       // (the Galerkin levels turn dense a few hundred rows above the 200-row target on large problems)
       // becomes the coarsest level
-      if (l == 0)
-        throw std::invalid_argument("smoothed aggregation: the aggregation of level 0 does not reduce it (" +
-                                    std::to_string(mats[l].cols) + " rows, " + std::to_string(n_agg) + " aggregates)");
+      if (l == 0) throw std::invalid_argument(sa_no_reduction_message(mats[l].cols, n_agg));
       break;
     }
     P.push_back(sa_prolongation(mats[l], agg, n_agg, l));
+    lap(t0, 1);
     Csc AH = galerkin(transpose(P.back()), mats[l], P.back());
     mats.push_back(std::move(AH));
+    lap(t0, 2);
   }
 }
 

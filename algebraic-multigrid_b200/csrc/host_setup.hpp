@@ -50,12 +50,22 @@ int64_t grid_lines(int64_t n);
 // (A.cols x n_agg).  Both throw std::invalid_argument naming `level` (and the row) on a zero diagonal;
 // sa_aggregate also on a strength threshold below 0 or NaN.
 int64_t sa_aggregate(const Csc& A, double theta, std::vector<int>& agg, int level = 0);
+// The two steps of sa_aggregate, so that the device setup (setup_sa.cuh builds the strength graph) runs the
+// same passes: sa_strength fills the strong-neighbour lists (CSR, ascending; same checks as sa_aggregate),
+// sa_aggregate_passes runs passes 1-3 on them.
+void sa_strength(const Csc& A, double theta, std::vector<int>& sptr, std::vector<int>& snb, int level = 0);
+int64_t sa_aggregate_passes(int n, const int* sptr, const int* snb, std::vector<int>& agg);
+// the std::invalid_argument messages of a zero diagonal and of a level 0 that does not reduce
+std::string sa_zero_diagonal_message(int level, int row);
+std::string sa_no_reduction_message(int rows, int64_t n_agg);
 Csc sa_prolongation(const Csc& A, const std::vector<int>& agg, int64_t n_agg, int level = 0);
 // The levels: mats[0] = A, then P[l] and mats[l + 1] = R (A P) with R = P^T while l + 1 < n_levels and
 // level l has more than kSaMaxCoarse rows.  A coarse level whose aggregation does not reduce it ends the
-// hierarchy as its coarsest level; when level 0 does not reduce, std::invalid_argument.
+// hierarchy as its coarsest level; when level 0 does not reduce, std::invalid_argument.  phase_s, when
+// given, accumulates the seconds spent in [aggregation, prolongators, Galerkin products].
 constexpr int kSaMaxCoarse = 200;
-void sa_hierarchy(Csc&& A, double theta, int n_levels, std::vector<Csc>& mats, std::vector<Csc>& P);
+void sa_hierarchy(Csc&& A, double theta, int n_levels, std::vector<Csc>& mats, std::vector<Csc>& P,
+                  double* phase_s = nullptr);
 // Eigen 3.4.0 conservative ColMajor product: entry (i,j) = sum over ascending k
 // of L(i,k)*R(k,j); numerical zeros kept; result columns sorted.
 Csc multiply(const Csc& L, const Csc& R);

@@ -11,7 +11,8 @@ reducing: that one is the coarsest), damped Jacobi 2+2 with fast
 arithmetic, PCG preconditioned by one V-cycle to ||b - A u|| / ||b|| <= 1e-8 from u = 0 with a seeded
 random right-hand side.  Each line: levels, operator complexity (sum of the levels' stored entries over
 level 0's), setup seconds (host clock around the constructor: aggregation, P, Galerkin products and the
-device mirrors, all host setup), ms per V-cycle (CUDA events over 30 graph replays after warm-up),
+device mirrors; built on the GPU unless AMGB_HOST_SETUP=1, `device_setup` says which) with its phases
+(`setup_phases`: Multigrid.setup_times(), each phase ending in a stream synchronise), ms per V-cycle (CUDA events over 30 graph replays after warm-up),
 PCG iterations and seconds (host clock around solve_pcg, which ends in a stream synchronise), the final
 relative residual recomputed on the host with scipy, and the level-0 times of k_residual (kind 1),
 k_restrict_sa (kind 2) and k_prolong_add_sa (kind 3) with their algorithmic bytes over a device-to-device
@@ -76,7 +77,8 @@ def run(kind, m, levels, rel_tol, bw, info):
     nnz = [mg.nnz(l) for l in range(L)]
     out = {"config": "sa_pcg_" + kind, "n": m, "levels": L, "level_rows": [mg.get_n_dofs(l) for l in range(L)],
            "operator_complexity": sum(nnz) / nnz[0], "formats": [mg.format(l) for l in range(L)],
-           "setup_s": round(setup_s, 3), "pcg_iters": mg.iters_done, "reported_rel": mg.last_error,
+           "setup_s": round(setup_s, 3), "device_setup": mg.device_setup,
+           "setup_phases": {k: round(v, 3) for k, v in mg.setup_times().items()}, "pcg_iters": mg.iters_done, "reported_rel": mg.last_error,
            "host_rel_residual": rel, "converged": rel <= rel_tol, "time_to_tol_s": round(solve_s, 4)}
     out["ms_per_vcycle"] = ms_per_cycle(mg)
     out["launches_per_vcycle"] = mg.launches_per_vcycle()
