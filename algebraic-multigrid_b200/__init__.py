@@ -865,6 +865,8 @@ class Multigrid:
         return lib().amgb_hierarchy_matrix_bytes(self.h, level)
 
     def n_diagonals(self, level):
+        """Diagonals a fused leg streams per row: every diagonal of the DIA mirror, or the centre and
+        upper ones on a level whose register-streaming legs read a bitwise-symmetric operator."""
         return lib().amgb_hierarchy_n_diagonals(self.h, level)
 
     def gs_kernel(self, level):

@@ -1607,6 +1607,7 @@ struct amgb_hierarchy {
     unsigned mask = 0;
     int kind_down = 0;
     bool matrix_free = false;  // the level's operator was verified to be a constant five-point stencil
+    bool half = false;         // the level's operator was verified to be bitwise symmetric: legs stream its upper half
     // row-type dictionary (option fuse bit 7): one byte per row + the table of the level's distinct rows
     int dict_types = 0;
     DevBuf<unsigned char> tid;
@@ -1680,6 +1681,22 @@ struct amgb_hierarchy {
     if (hb) return false;
     for (int d = 0; d < 5; ++d) cst[d] = C.c[d];
     return true;
+  }
+  // Half-streaming legs: true when the square DIA mirror D is bitwise symmetric, A(r, r+o) == A(r+o, r) for
+  // every stored entry, and stores nothing outside the level (setup_dia.cuh)
+  bool check_symmetric(const DevDia& D) {
+    if (D.n_rows < 1 || D.n_diag < 1 || D.n_diag > setup::kMaxOffsets) return false;
+    setup::Offsets off{};
+    off.n = D.n_diag;
+    for (int d = 0; d < D.n_diag; ++d) off.v[d] = D.off[d];
+    DevBuf<int> flag;
+    flag.alloc(1);
+    flag.zero(stream);
+    LAUNCH(setup::k_dia_asymmetric, blocks_for(D.n_rows, 256), 256, 0, stream, D.val.p, D.n_rows, D.ld, off, flag.p);
+    int asym = 1;
+    CUDA_CHECK(cudaMemcpyAsync(&asym, flag.p, sizeof(int), cudaMemcpyDeviceToHost, stream));
+    CUDA_CHECK(cudaStreamSynchronize(stream));
+    return asym == 0;
   }
   // Row-type dictionary of a DIA mirror (option fuse bit 7): at most 256 distinct rows, every row
   // verified bit for bit against its table row.  Returns the number of types (0: not applicable).
@@ -1755,6 +1772,7 @@ struct amgb_hierarchy {
     if ((int)leg_side.size() != L) leg_side.assign(L, 0);
     LegLevel& G = legs[l];
     G.ok = false;
+    G.half = false;
     if (!(opt.fuse & 12) || opt.smoother != AMGB_SMOOTHER_JACOBI || opt.smoother_iters < 1 || l + 1 >= L) return;
     const LevelState& S = lv[l];
     if (!S.tmp.p) return;
@@ -1852,6 +1870,9 @@ struct amgb_hierarchy {
           G.matrix_free = mf;
           G.dict_types = mf ? 0 : build_dictionary(A.dia, G.tid, G.table);
           dummy.dict_types = G.dict_types;
+          // sharded levels (branch above) stream every diagonal: their ghost rows would need one more operator line
+          G.half = !mf && G.dict_types == 0 && check_symmetric(A.dia);
+          dummy.half = G.half;
           auto plan = [&](int kind, int NS, int X) {
             int wps = 12;
             sleg_dispatch(kind, mask, dummy, nullptr, 2, &wps);
@@ -1883,6 +1904,7 @@ struct amgb_hierarchy {
             // level 0 down leg 231 -> 197 us, profiles/r2_stream_legs.md) and costs issue slots below
             P.l2_ahead = env_int("AMGB_SLEG_L2AHEAD", n[l] >= (1 << 21) ? 2 : 0);
             P.matrix_free = mf;
+            P.half = G.half;
             for (int d = 0; d < 5; ++d) P.cst[d] = cst[d];
             P.finish(A.dia.n_diag);
             return P;
@@ -4285,11 +4307,14 @@ int amgb_hierarchy_format(const amgb_hierarchy* h, int level) {
   if (!h || level < 0 || level >= h->L) return -1;
   return h->ops[level]->rows_of_A().is_dia ? AMGB_FORMAT_DIA : AMGB_FORMAT_SELL;
 }
-// diagonals of the level's DIA mirror (0 for SELL): what a fused leg streams is 8 x diagonals bytes per row
+// diagonals a fused leg streams from the level's DIA mirror (0 for SELL), 8 bytes per row each: all of
+// them, or the centre and upper ones on a half-streamed level
 int amgb_hierarchy_n_diagonals(const amgb_hierarchy* h, int level) {
   if (!h || level < 0 || level >= h->L) return -1;
   const DevMat& A = h->ops[level]->rows_of_A();
-  return A.is_dia ? A.dia.n_diag : 0;
+  if (!A.is_dia) return 0;
+  if (h->leg_ok(level) && h->legs[level].stream && h->legs[level].half) return A.dia.n_diag / 2 + 1;
+  return A.dia.n_diag;
 }
 int amgb_hierarchy_gs_kernel(const amgb_hierarchy* h, int level) {
   if (!h || level < 0 || level >= h->L || h->opt.smoother != AMGB_SMOOTHER_GS) return -1;

@@ -20,9 +20,9 @@ int env_int(const char* name, int dflt) {
   return v ? std::atoi(v) : dflt;
 }
 
-template <int KIND, unsigned MASK, int NU, int PF, bool FAST>
+template <int KIND, unsigned MASK, int NU, int PF, bool FAST, bool HALF>
 bool act(const Params& P, cudaStream_t s, int action, int* warps_per_sm) {
-  auto kern = k_stream_leg<KIND, MASK, NU, PF, FAST>;
+  auto kern = k_stream_leg<KIND, MASK, NU, PF, FAST, HALF>;
   if (action == 1) {
     kern<<<(P.n_warps + 3) / 4, 128, 0, s>>>(P);
     check(cudaGetLastError(), "k_stream_leg launch");
@@ -67,6 +67,18 @@ bool act_dict(const Params& P, cudaStream_t s, int action, int* warps_per_sm) {
   return true;
 }
 
+template <int KIND, unsigned MASK, bool FAST, bool HALF>
+bool by_pf(const Params& P, cudaStream_t s, int action, int* wps) {
+  if (P.nu == 1) return act<KIND, MASK, 1, 2, FAST, HALF>(P, s, action, wps);
+  if (P.nu != 2) return false;
+  // five-point up leg: three lines in flight at 12 warps/SM measured 6 % faster than two at 16
+  // (reference-order arithmetic, profiles/r1_stream_legs.md); AMGB_SLEG_PF overrides
+  if constexpr (MASK == kMask5) {
+    if (env_int("AMGB_SLEG_PF", (KIND == UP && !FAST) ? 3 : 2) == 3) return act<KIND, MASK, 2, 3, FAST, HALF>(P, s, action, wps);
+  }
+  return act<KIND, MASK, 2, 2, FAST, HALF>(P, s, action, wps);
+}
+
 template <int KIND, unsigned MASK, bool FAST>
 bool by_nu(const Params& P, cudaStream_t s, int action, int* wps) {
   if (P.dict_types > 0) {
@@ -82,14 +94,7 @@ bool by_nu(const Params& P, cudaStream_t s, int action, int* wps) {
       return false;
     }
   }
-  if (P.nu == 1) return act<KIND, MASK, 1, 2, FAST>(P, s, action, wps);
-  if (P.nu != 2) return false;
-  // five-point up leg: three lines in flight at 12 warps/SM measured 6 % faster than two at 16
-  // (reference-order arithmetic, profiles/r1_stream_legs.md); AMGB_SLEG_PF overrides
-  if constexpr (MASK == kMask5) {
-    if (env_int("AMGB_SLEG_PF", (KIND == UP && !FAST) ? 3 : 2) == 3) return act<KIND, MASK, 2, 3, FAST>(P, s, action, wps);
-  }
-  return act<KIND, MASK, 2, 2, FAST>(P, s, action, wps);
+  return P.half ? by_pf<KIND, MASK, FAST, true>(P, s, action, wps) : by_pf<KIND, MASK, FAST, false>(P, s, action, wps);
 }
 
 template <int KIND, bool FAST>

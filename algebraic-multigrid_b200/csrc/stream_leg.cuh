@@ -35,6 +35,15 @@
 // garbage.  No existing row reads them with a non-zero coefficient (the operator has no entry
 // there), and 0 * finite = 0, so the results of the rows that are stored are unaffected.
 //
+// Half streaming (template flag HALF, Params::half): on a level whose operator is bitwise symmetric
+// the kernel loads only the centre and upper slots 4..8 of each row.  A lower coefficient is the
+// upper coefficient of the row it couples to, a(k, k+o) = a(k+o, k) for o = a*m + delta < 0, and
+// that row sits on lane i + delta of the previous line (a = -1) or of the same line (slot 3): it is
+// taken from registers by a shuffle when the line enters the input stage, where the ring still
+// holds the previous line (one extra line is loaded before the loop for the first one).  The
+// coefficient bits and the summation order do not change.  Rows k + o < 0 get an explicit 0: the
+// previous line of line 0 was loaded clamped and holds row 0's non-zero upper coefficients.
+//
 // Multi-GPU (Params::sync.enabled): the edge warps wait for the neighbour's previous site before
 // touching ghost rows and push their boundary rows into the neighbour's ghost rows at the end
 // (stream_leg_api.hpp, struct Sync) -- the halo exchange costs no launch.
@@ -60,10 +69,13 @@ __device__ __forceinline__ double rcp_refined(double d) {
 // MF: matrix-free five-point operator (Params::cst, presence of a neighbour decided from the row index)
 // DICT: the operator row comes from a table of the level's distinct rows in shared memory, selected
 //       by one byte per row (Params::tid / table) -- 1 instead of 8 x diagonals bytes per row from HBM
-template <int KIND, unsigned MASK, int NU, int PF_, bool FAST, bool MF = false, bool DICT = false>
+// HALF: only the centre and upper slots are loaded, the lower ones are derived (bitwise-symmetric operator)
+template <int KIND, unsigned MASK, int NU, int PF_, bool FAST, bool MF = false, bool DICT = false, bool HALF = false>
 struct Leg {
   static_assert(!(MF && DICT), "one operator source");
   static_assert(!MF || MASK == kMask5, "the matrix-free variant is the five-point stencil");
+  static_assert(!HALF || (!MF && !DICT), "half streaming reads the DIA mirror");
+  static_assert(!HALF || mirror9(MASK) == MASK, "half streaming needs slot 8 - SL for every lower slot SL");
   static constexpr int ND = popc9(MASK);
   static constexpr int NS = stages(KIND, NU);                // chained stencil stages
   static constexpr int H = lost_lanes(KIND, NU);             // lanes lost on each side
@@ -72,6 +84,10 @@ struct Leg {
   static constexpr int DC = popc9(MASK & 0xFu);              // rank of the centre slot (0,0)
   static constexpr int S_OUT = (KIND == UP) ? NS : NS - 1;   // stage whose result is the iterate
   static_assert((MASK >> 4) & 1u, "the diagonal must be present");
+  // derived coefficients of lane 0 (delta = -1) and lane 31 (delta = +1) are garbage: those lanes
+  // must be lost after the first stencil stage already
+  static_assert(!HALF || H >= 1, "half streaming needs the edge lanes lost");
+  static constexpr int D0 = HALF ? DC : 0;  // first operator slot loaded from memory
 
   struct Line {
     double a[MF ? 1 : ND];  // operator row (not loaded by the matrix-free variant)
@@ -116,6 +132,11 @@ struct Leg {
     return (unsigned)(Jl - P.e_lo) < (unsigned)P.e_cnt;
   }
 
+  // the operator slots that come from memory (row index already clamped)
+  static __device__ __forceinline__ void load_row(Line& L, const Params& P, int kc) {
+#pragma unroll
+    for (int d = D0; d < ND; ++d) L.a[d] = __ldg(P.vd[d] + kc);
+  }
   // loads of the line whose row on this lane is k (clamped to the rows that exist)
   static __device__ __forceinline__ void load(Line& L, const Params& P, int k, const double* table = nullptr) {
     const int kc = min(max(k, P.row_lo), P.row_hi1);
@@ -124,8 +145,7 @@ struct Leg {
 #pragma unroll
       for (int d = 0; d < ND; ++d) L.a[d] = row[d];
     } else if constexpr (!MF) {
-#pragma unroll
-      for (int d = 0; d < ND; ++d) L.a[d] = __ldg(P.vd[d] + kc);
+      load_row(L, P, kc);
     }
     L.f = __ldg(P.f + kc);
     if (KIND != DOWN_ZERO) L.u = __ldg(P.uin + kc);
@@ -145,7 +165,7 @@ struct Leg {
     const int kc = min(max(k, P.row_lo), P.row_hi1);
     if constexpr (!MF && !DICT) {
 #pragma unroll
-      for (int d = 0; d < ND; ++d) asm volatile("prefetch.global.L2 [%0];" ::"l"(P.vd[d] + kc));
+      for (int d = D0; d < ND; ++d) asm volatile("prefetch.global.L2 [%0];" ::"l"(P.vd[d] + kc));
     }
     asm volatile("prefetch.global.L2 [%0];" ::"l"(P.f + kc));
     if (KIND != DOWN_ZERO) asm volatile("prefetch.global.L2 [%0];" ::"l"(P.uin + kc));
@@ -171,6 +191,28 @@ struct Leg {
       }
       return __dadd_rn(L.u, acc);
     }
+  }
+
+  // HALF: lower slot SL of line L (global row kg on this lane) from upper slot 8 - SL of row kg + o,
+  // o = a * m + delta: lane i + delta of the previous line Lp (a = -1) or of L itself (a = 0)
+  template <int SL>
+  static __device__ __forceinline__ void derive_slot(Line& L, const Line& Lp, int m, int kg) {
+    if constexpr (SL < 4 && ((MASK >> SL) & 1u)) {
+      constexpr int d = popc9(MASK & ((1u << SL) - 1u));
+      constexpr int du = popc9(MASK & ((1u << (8 - SL)) - 1u));
+      constexpr int a = SL / 3 - 1, dl = SL % 3 - 1;
+      const double src = (a < 0) ? Lp.a[du] : L.a[du];
+      double v = src;
+      if constexpr (dl < 0) v = __shfl_up_sync(0xffffffffu, src, 1);
+      if constexpr (dl > 0) v = __shfl_down_sync(0xffffffffu, src, 1);
+      L.a[d] = (kg + a * m + dl >= 0) ? v : 0.0;  // the row before the level start was loaded clamped
+    }
+  }
+  static __device__ __forceinline__ void derive(Line& L, const Line& Lp, int m, int kg) {
+    derive_slot<0>(L, Lp, m, kg);
+    derive_slot<1>(L, Lp, m, kg);
+    derive_slot<2>(L, Lp, m, kg);
+    derive_slot<3>(L, Lp, m, kg);
   }
 
   template <int SL, class Row>
@@ -246,6 +288,9 @@ struct Leg {
   template <int P_>
   static __device__ __forceinline__ void step(State& S, const Params& P, int k1, const Own& own, const Lane& Z) {
     const int m = P.m;
+    // lower slots of line jj + 1 from line jj (slot P_ - 1, still in the ring); ahead of the ring load,
+    // which measured fewer spills in the reference-order nine-point legs
+    if constexpr (HALF) derive(S.R[P_ % RS], S.R[(P_ + RS - 1) % RS], m, k1 + P.base);
     load(S.R[(P_ + PF) % RS], P, k1 + PF * m, Z.table);
     if (P.l2_ahead > 0) prefetch(P, k1 + (PF + P.l2_ahead) * m);
     // ---- input stage, line jj + 1
@@ -456,6 +501,8 @@ struct Leg {
     }
 #pragma unroll
     for (int q = 0; q < PF; ++q) load(S.R[q], P, k1 + q * P.m, Z.table);
+    // the line before jA, whose upper slots give jA its lower ones (slot RS - 1 is first loaded at step NS)
+    if constexpr (HALF) load_row(S.R[RS - 1], P, min(max(k1 - P.m, P.row_lo), P.row_hi1));
     if (!waits) {
       // single GPU: the plain line loop (its own copy, so the multi-GPU bookkeeping below costs it nothing);
       // its trip count is a kernel parameter, i.e. provably uniform
@@ -480,10 +527,10 @@ struct Leg {
   }
 };
 
-template <int KIND, unsigned MASK, int NU, int PF_, bool FAST>
+template <int KIND, unsigned MASK, int NU, int PF_, bool FAST, bool HALF>
 __global__ void __launch_bounds__(128, (popc9(MASK) <= 5 && PF_ == 2) ? 4 : 3)
     k_stream_leg(const __grid_constant__ Params P) {
-  Leg<KIND, MASK, NU, PF_, FAST>::run(P);
+  Leg<KIND, MASK, NU, PF_, FAST, false, false, HALF>::run(P);
 }
 // row-type dictionary legs (at most 256 distinct operator rows on the level)
 template <int KIND, unsigned MASK, int NU, bool FAST>

@@ -89,6 +89,9 @@ struct Params {
   int dict_types;              // 0: off
   const unsigned char* tid;    // type of every row of the window
   const double* table;         // dict_types x (number of diagonals)
+  // half streaming (the operator was VERIFIED to be bitwise symmetric): only vd[] of the centre and
+  // upper diagonals are read, the lower coefficients come from registers
+  int half;
   double omega;
   const double* val;
   const double* vd[9];  // val + d * ld
@@ -152,6 +155,12 @@ __host__ __device__ constexpr int popc9(unsigned v) {
   for (int i = 0; i < 9; ++i) c += (v >> i) & 1u;
   return c;
 }
+// slot mask mirrored through the centre (slot sl -> 8 - sl: offset o -> -o)
+__host__ __device__ constexpr unsigned mirror9(unsigned v) {
+  unsigned r = 0;
+  for (int i = 0; i < 9; ++i) r |= ((v >> i) & 1u) << (8 - i);
+  return r;
+}
 // lanes lost on each side of a warp: one per chained stencil stage (+ 1 for the restriction)
 __host__ __device__ constexpr int stages(int kind, int nu) { return kind == DOWN_U ? nu + 1 : nu; }
 __host__ __device__ constexpr int lost_lanes(int kind, int nu) { return stages(kind, nu) + (kind == UP ? 0 : 1); }
@@ -160,7 +169,8 @@ __host__ __device__ constexpr int lost_lanes(int kind, int nu) { return stages(k
 // `s` (returns true when a kernel was launched).  2: set the L1 carve-out (outside stream capture)
 // and report the resident warps per SM the register count allows in *warps_per_sm.
 // fast: AMGB_ARITH_FAST kernels (FMA + refined reciprocal) instead of the reference-order ones.
-// Params::matrix_free selects the matrix-free five-point kernels (kMask5 only).
+// Params::matrix_free selects the matrix-free five-point kernels (kMask5 only), Params::half the
+// half-streaming ones.
 bool dispatch(int kind, unsigned mask, const Params& P, cudaStream_t s, int action, int* warps_per_sm, bool fast);
 
 }  // namespace sleg
