@@ -142,6 +142,7 @@ SIGNATURES = {
     "amgb_solve": (_i, [_p, C.POINTER(_l), C.POINTER(_d)]),
     "amgb_solve_relative": (_i, [_p, _d, C.POINTER(_l), C.POINTER(_d)]),
     "amgb_solve_pcg": (_i, [_p, _d, _l, C.POINTER(_l), C.POINTER(_d)]),
+    "amgb_solve_gmres": (_i, [_p, _d, _i, _l, C.POINTER(_l), C.POINTER(_d)]),
     "amgb_hierarchy_iters_done": (_l, [_p]),
     "amgb_hierarchy_error_history": (_l, [_p, _pd, _l]),
     "amgb_synchronize": (_i, [_p]),
@@ -790,6 +791,14 @@ class Multigrid:
         """Conjugate gradients preconditioned by one V-cycle (beyond the reference)."""
         it, rel = _l(), _d()
         _check(lib().amgb_solve_pcg(self.h, rel_tol, max_iters, C.byref(it), C.byref(rel)))
+        self.iters_done, self.last_error = it.value, rel.value
+        return self.get_soln(0)
+
+    def solve_gmres(self, rel_tol, restart=30, max_iters=1000):
+        """Restarted GMRES(restart) right-preconditioned by one V-cycle, for symmetric and unsymmetric A alike
+        (beyond the reference).  iters_done counts Arnoldi steps; last_error is the true relative residual."""
+        it, rel = _l(), _d()
+        _check(lib().amgb_solve_gmres(self.h, rel_tol, restart, max_iters, C.byref(it), C.byref(rel)))
         self.iters_done, self.last_error = it.value, rel.value
         return self.get_soln(0)
 

@@ -28,6 +28,7 @@
 #include "galerkin_dia2d.cuh"
 #include "gs_wave.cuh"
 #include "kernels.cuh"
+#include "krylov.cuh"
 #include "line_gs.cuh"
 #include "mid_levels.cuh"
 #include "setup_dia.cuh"
@@ -4005,6 +4006,151 @@ int amgb_solve_pcg(amgb_hierarchy* h, double rel_tol, int64_t max_iters, int64_t
     CUDA_CHECK(cudaStreamSynchronize(s));
     h->iters_done = iter;
     if (iters_done) *iters_done = iter;
+    if (last_rel_residual) *last_rel_residual = rel;
+  });
+}
+// Restarted GMRES(m) on A x = b right-preconditioned by one V-cycle from a zero guess (M(v)), so the
+// monitored quantity is the true residual.  Arnoldi with classical Gram-Schmidt and one
+// reorthogonalisation on the device (krylov.cuh); the Hessenberg column, its Givens rotations and the
+// back substitution on the host.  Specification: include/amgb.h, tests/oracle_gmres.py.
+int amgb_solve_gmres(amgb_hierarchy* h, double rel_tol, int restart, int64_t max_iters, int64_t* iters_done,
+                     double* last_rel_residual) {
+  return guarded([&] {
+    if (!h) throw std::invalid_argument("null argument");
+    if (!(rel_tol >= 0.0)) throw std::invalid_argument("amgb_solve_gmres: rel_tol must be >= 0");
+    if (restart < 1) throw std::invalid_argument("amgb_solve_gmres: restart must be >= 1");
+    if (max_iters < 0) throw std::invalid_argument("amgb_solve_gmres: max_iters must be >= 0");
+    if (h->lv[0].sharded) throw ApiError(AMGB_ESTATE, "amgb_solve_gmres runs on a single GPU");
+    CUDA_CHECK(cudaSetDevice(h->device));
+    cudaStream_t s = h->stream;
+    LevelState& S = h->lv[0];
+    const int64_t N = h->n[0];
+    const size_t bytes = sizeof(double) * (size_t)N;
+    const int m = restart;
+    const int64_t ld = krylov::basis_ld(N);
+    const int nb = krylov::tiles(N), nbv = std::max(1, blocks_for(N, krylov::kThreads));
+    DevBuf<double> b, x, zero;
+    for (DevBuf<double>* v : {&b, &x, &zero}) v->alloc((size_t)N + 8);
+    zero.zero(s);
+    CUDA_CHECK(cudaMemcpyAsync(b.p, S.f.p, bytes, cudaMemcpyDeviceToDevice, s));
+    CUDA_CHECK(cudaMemcpyAsync(x.p, S.u.p, bytes, cudaMemcpyDeviceToDevice, s));
+    auto sumsq = [&](const double* v) {
+      LAUNCH(dev::k_sumsq_partial, nbv, 256, 0, s, v, (int)N, h->partial.p);
+      LAUNCH(dev::k_sum_partials, 1, 256, 0, s, h->partial.p, nbv, h->scalar.p);
+      return h->finish_scalar_local();
+    };
+    const double bnorm = std::sqrt(sumsq(b.p));
+    h->history.clear();
+    int64_t it = 0;
+    double rel = 0.0;
+    if (bnorm > 0.0) {
+      // the (m + 1) x ld basis, the k x nb dot partials and one Hessenberg column (h, h', |w|^2)
+      DevBuf<double> V, part, col;
+      {
+        const double want = (double)(m + 1) * (double)ld * sizeof(double);
+        cudaError_t e = want < 9.0e18 ? cudaMalloc(&V.p, (size_t)(m + 1) * (size_t)ld * sizeof(double))
+                                      : cudaErrorMemoryAllocation;
+        if (e != cudaSuccess) {
+          cudaGetLastError();
+          V.p = nullptr;
+          throw ApiError(AMGB_ECUDA, "amgb_solve_gmres: cannot allocate the Krylov basis of " +
+                                         std::to_string(m + 1) + " x " + std::to_string(N) + " doubles (" +
+                                         std::to_string(want / 1e9) + " GB): " + cudaGetErrorString(e));
+        }
+        V.n = (size_t)(m + 1) * (size_t)ld;
+      }
+      part.alloc((size_t)m * nb);
+      col.alloc(2 * (size_t)m + 1);
+      auto vec = [&](int i) { return V.p + (size_t)i * ld; };
+      std::vector<double> H((size_t)(m + 1) * m), cs(m), sn(m), g(m + 1), y(m), hcol(2 * (size_t)m + 1);
+      auto Hij = [&](int i, int j) -> double& { return H[(size_t)j * (m + 1) + i]; };
+      // r = b - A x into v_0; the true relative residual
+      auto true_residual = [&]() {
+        h->ops[0]->residual(x.p, b.p, vec(0), s);
+        return std::sqrt(sumsq(vec(0)));
+      };
+      double beta = true_residual();
+      rel = beta / bnorm;
+      bool failed = false;
+      while (!failed && it < max_iters && rel > rel_tol) {
+        LAUNCH(krylov::k_scale, nbv, krylov::kThreads, 0, s, vec(0), vec(0), beta, N);
+        std::fill(g.begin(), g.end(), 0.0);
+        g[0] = beta;
+        int k = 0;  // Arnoldi steps of this cycle
+        for (int j = 0; j < m && it < max_iters; ++j) {
+          // w = A M(v_j) into v_{j+1}: a cycle on -v_j, then 0 - A z
+          LAUNCH(krylov::k_negate, nbv, krylov::kThreads, 0, s, S.f.p, vec(j), N);
+          CUDA_CHECK(cudaMemsetAsync(S.u.p, 0, bytes, s));
+          h->vcycle();
+          double* w = vec(j + 1);
+          h->ops[0]->residual(S.u.p, zero.p, w, s);
+          const int kk = j + 1;
+          LAUNCH(krylov::k_multidot, nb, krylov::kThreads, 0, s, V.p, ld, kk, w, N, part.p);
+          LAUNCH(krylov::k_sum_rows, kk, krylov::kThreads, 0, s, part.p, nb, col.p);
+          LAUNCH(krylov::k_update<krylov::kDots>, nb, krylov::kThreads, 0, s, w, w, V.p, ld, kk, col.p, N, part.p);
+          LAUNCH(krylov::k_sum_rows, kk, krylov::kThreads, 0, s, part.p, nb, col.p + kk);
+          LAUNCH(krylov::k_update<krylov::kSumSq>, nb, krylov::kThreads, 0, s, w, w, V.p, ld, kk, col.p + kk, N,
+                 part.p);
+          LAUNCH(krylov::k_sum_rows, 1, krylov::kThreads, 0, s, part.p, nb, col.p + 2 * kk);
+          CUDA_CHECK(cudaMemcpyAsync(hcol.data(), col.p, sizeof(double) * (2 * kk + 1), cudaMemcpyDeviceToHost, s));
+          CUDA_CHECK(cudaStreamSynchronize(s));
+          bool finite = true;
+          for (int i = 0; i < kk; ++i) {
+            Hij(i, j) = hcol[i] + hcol[kk + i];
+            finite = finite && std::isfinite(Hij(i, j));
+          }
+          const double hnext = std::sqrt(hcol[2 * kk]);
+          Hij(j + 1, j) = hnext;
+          if (!finite || !std::isfinite(hnext)) {  // abandon the cycle: x stays that of the last one
+            failed = true;
+            break;
+          }
+          if (hnext != 0.0) LAUNCH(krylov::k_scale, nbv, krylov::kThreads, 0, s, w, w, hnext, N);
+          for (int i = 0; i < j; ++i) {
+            const double t = cs[i] * Hij(i, j) + sn[i] * Hij(i + 1, j);
+            Hij(i + 1, j) = -sn[i] * Hij(i, j) + cs[i] * Hij(i + 1, j);
+            Hij(i, j) = t;
+          }
+          const double d = std::hypot(Hij(j, j), hnext);
+          if (d == 0.0) {  // A M v_j = 0: singular, no rotation
+            failed = true;
+            break;
+          }
+          cs[j] = Hij(j, j) / d;
+          sn[j] = hnext / d;
+          Hij(j, j) = d;
+          Hij(j + 1, j) = 0.0;
+          g[j + 1] = -sn[j] * g[j];
+          g[j] = cs[j] * g[j];
+          k = j + 1;
+          it += 1;
+          const double est = std::fabs(g[j + 1]) / bnorm;
+          h->history.push_back(est);
+          if (est <= rel_tol || hnext == 0.0) break;
+        }
+        if (failed || k == 0) break;
+        // y = H(0:k, 0:k) \ g(0:k); t = V_k y (c = -y from a zero base) into f_0; x += M(t)
+        for (int i = k - 1; i >= 0; --i) {
+          double acc = g[i];
+          for (int q = i + 1; q < k; ++q) acc -= Hij(i, q) * y[q];
+          y[i] = acc / Hij(i, i);
+        }
+        for (int i = 0; i < k; ++i) hcol[i] = -y[i];
+        CUDA_CHECK(cudaMemcpyAsync(col.p, hcol.data(), sizeof(double) * k, cudaMemcpyHostToDevice, s));
+        LAUNCH(krylov::k_update<krylov::kNone>, nb, krylov::kThreads, 0, s, S.f.p, nullptr, V.p, ld, k, col.p, N,
+               nullptr);
+        CUDA_CHECK(cudaMemsetAsync(S.u.p, 0, bytes, s));
+        h->vcycle();
+        LAUNCH(dev::k_axpy, nbv, 256, 0, s, x.p, 1.0, S.u.p, (int)N);
+        beta = true_residual();
+        rel = beta / bnorm;
+      }
+    }
+    CUDA_CHECK(cudaMemcpyAsync(S.f.p, b.p, bytes, cudaMemcpyDeviceToDevice, s));
+    CUDA_CHECK(cudaMemcpyAsync(S.u.p, x.p, bytes, cudaMemcpyDeviceToDevice, s));
+    CUDA_CHECK(cudaStreamSynchronize(s));
+    h->iters_done = it;
+    if (iters_done) *iters_done = it;
     if (last_rel_residual) *last_rel_residual = rel;
   });
 }

@@ -163,6 +163,16 @@ class Multigrid {
     last_error_ = rel;
     return get_soln(0);
   }
+  // Restarted GMRES(restart) right-preconditioned by one V-cycle, for unsymmetric A as well (amgb.h,
+  // amgb_solve_gmres); iterations_done() counts Arnoldi steps, last_error() is the true relative residual.
+  const VectorT<EleType>& solve_gmres(EleType rel_tol, int restart = 30, size_t max_iters = 1000) {
+    int64_t it = 0;
+    double rel = 0;
+    detail::check(amgb_solve_gmres(h, rel_tol, restart, (int64_t)max_iters, &it, &rel));
+    iters_done_ = (size_t)it;
+    last_error_ = rel;
+    return get_soln(0);
+  }
   amgb_hierarchy* handle() { return h; }
   size_t get_n_levels() const { return n_levels; }
 
